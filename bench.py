@@ -18,6 +18,9 @@ process per GPU; C2's single stream is replicated per rank, stream lists are sha
 the process group is gloo and only carries barriers, timings and result lists).
 `--impl reference` times the CPU restatement of the reference (oracle/, the reference itself is Java and this image
 has no JVM) with every host core on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the last timed step computed as .npy files (dump_outputs).  The inputs come from fixed
+seeds, so two builds run with the same arguments can be compared output for output (`--workload ref` also sizes its
+sample by the host's core count).
 """
 import argparse
 import ctypes as C
@@ -33,6 +36,7 @@ import time
 import zlib
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the tree may be read-only: the benchmark writes nothing into it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -60,7 +64,14 @@ def parse_args():
     ap.add_argument("--no-shapes", action="store_true", help="skip the short C3/C4/C5 runs")
     ap.add_argument("--no-verify", action="store_true", help="skip inflating the output of the last timed step")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed as DIR/<name>.npy (see dump_outputs)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
+    return a
 
 
 def workload_config(a):
@@ -363,9 +374,10 @@ class Ctx:
         return sum(self.gather(x))
 
 
-def measure(ctx, L, N, streams, merge, steps, warmup, sample_clocks=False, verify=False, e2e_steps=None):
+def measure(ctx, L, N, streams, merge, steps, warmup, sample_clocks=False, verify=False, e2e_steps=None, dump=None):
     """value (device-resident, CUDA events on the launching stream), e2e (pinned host buffers through the batch
-    entry), kernel-family times, launches, output verification — for this rank's `streams`."""
+    entry), kernel-family times, launches, output verification — for this rank's `streams`.  With `dump`, the results
+    of the last timed step are written there (dump_outputs)."""
     torch = ctx.torch
     n = len(streams)
     in_bytes = sum(len(s) for s in streams)
@@ -420,6 +432,8 @@ def measure(ctx, L, N, streams, merge, steps, warmup, sample_clocks=False, verif
         out["out_bytes"] = sum(r.out_len for r in res)
         out["unc_bytes"] = sum(r.uncompressed_len for r in res)
         out["saved_bits"] = sum(r.saved_bits for r in res)
+        if dump:
+            dump_outputs(dump, N, res)
         if verify:
             t0 = time.time()
             drift = 0
@@ -476,6 +490,38 @@ def verify_stream(raw, opt, r):
     # saved_bits is the reference's own running count (DeflateStream.java:519,565); with stored blocks it follows the
     # drifting `pos` (SURVEY.md H5), so it is reported, not asserted
     return r.size_bits_in - r.size_bits_out - r.saved_bits
+
+
+DUMP_BYTES = 1 << 23     # output bytes kept by dump_outputs (32 MB as float32)
+DUMP_SEED = 0xD4D0
+
+
+def dump_outputs(path, N, res):
+    """Write what a caller of the timed path receives for every stream, in stream order, as float64 `<field>.npy`
+    (every field of deft4cu_result except the output buffer itself), plus `out_crc32.npy` (CRC-32 of each output
+    stream: covers every byte) and `out_bytes.npy` (float32).  `out_bytes` is all output streams concatenated when they
+    hold at most DUMP_BYTES bytes, otherwise the bytes at the sorted positions
+    np.random.default_rng(DUMP_SEED).integers(0, total_length, DUMP_BYTES): the same positions whenever the total
+    length is the same."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    views = [np.ctypeslib.as_array(r.out, (r.out_len,)) if r.out_len else np.zeros(0, np.uint8) for r in res]
+    for name, _ in N.Result._fields_:
+        if name != "out":
+            np.save(os.path.join(path, name + ".npy"), np.array([getattr(r, name) for r in res], dtype=np.float64))
+    np.save(os.path.join(path, "out_crc32.npy"), np.array([zlib.crc32(v) for v in views], dtype=np.float64))
+    starts = np.cumsum([0] + [len(v) for v in views])
+    total = int(starts[-1])
+    if total <= DUMP_BYTES:
+        pos = np.arange(total)
+    else:
+        pos = np.sort(np.random.default_rng(DUMP_SEED).integers(0, total, DUMP_BYTES))
+    sample = np.empty(len(pos), np.float32)
+    bounds = np.searchsorted(pos, starts)
+    for k, v in enumerate(views):
+        lo, hi = bounds[k], bounds[k + 1]
+        sample[lo:hi] = v[pos[lo:hi] - starts[k]]
+    np.save(os.path.join(path, "out_bytes.npy"), sample)
 
 
 def roofline_of(m, peak, peak_src):
@@ -656,7 +702,10 @@ def run_ours(a):
     t_gen = time.time()
     streams = make_streams(a, ctx.rank)
     t_gen = time.time() - t_gen
-    m = measure(ctx, L, N, streams, merge, a.steps, a.warmup, sample_clocks=True, verify=not a.no_verify)
+    dump = a.dump_outputs
+    if dump and ctx.world > 1:
+        dump = os.path.join(dump, "rank%d" % ctx.rank)
+    m = measure(ctx, L, N, streams, merge, a.steps, a.warmup, sample_clocks=True, verify=not a.no_verify, dump=dump)
     dev_ms = ctx.max(m["dev_ms"])
     total_in = ctx.sum(m["in_bytes"])
     value = total_in * a.steps / (dev_ms / 1e3) / 1e6
