@@ -3,7 +3,7 @@
 // One CTA owns one block.  Thread 0 sweeps the enumeration of DeflateStream.optimiseBlock (DeflateStream.java:343-490)
 // over memo tables in shared memory; every miss becomes a request.  After a sweep the whole CTA computes the requests:
 //   passes   replaceBackrefsWithLiteralsIfSmaller / removeDistLitLeastExpensive (DeflateBlockHuffman.java:222-319,
-//            373-458): CTA-wide, 8 symbols per thread, against a per-table cost array dc[i] = literal cost - match cost.
+//            373-458): CTA-wide, 8 matches per thread, against a per-table cost array dc[j] = literal cost - match cost.
 //            The cost array of a table is built in ONE coalesced pass over the block's decoded bytes: 2 KiB tiles, per-byte
 //            code lengths looked up in shared memory, a CTA-wide prefix sum per tile, every match takes P[end] - P[start].
 //   recodes  recodeHuffman (:670-743): one WARP per request - histogram row -> litlen and distance Huffman trees with the
@@ -12,6 +12,9 @@
 //   headers  recodeHeader / recodeHeaderToLessRLEMatches / optimiseHeader (:471-476,579-635): one warp per request.
 //   trials   the 56 header strategies of a table (DeflateStream.java:277-316): 28 threads per table, 8 tables at a time,
 //            sizes only (huff.cuh trial_sizes); the winner alone is materialised.
+// Inside the engine a block is its matches: match j is the j-th match in symbol order, and every per-block array (masks,
+// cost arrays, sign masks, match records) is indexed by j, since literals never change.  The mask pool outside the engine
+// keeps one bit per symbol; load_block and store_mask translate.
 // Masks (symbol lists), Tabs and Hdrs are immutable entries of per-CTA pools in global scratch, hash-consed where it
 // pays (masks, Tabs); a pool that fills up makes the round restart in segments with a reset between them.
 #pragma once
@@ -50,7 +53,8 @@ struct BlkView {
     const uint32_t* symout;
     const uint8_t* out;
     uint32_t n;       // symbols (including NOPs left by a merge)
-    uint32_t nwords;  // mask words
+    uint32_t nm;      // matches (build_views)
+    uint32_t nwords;  // mask words: the engine's masks have one bit per match (build_views)
     uint64_t ulen;    // decoded length
     uint64_t out_off; // pool offset of the block's first decoded byte
 };
@@ -134,24 +138,27 @@ struct EngScratch {
     unsigned char* slab;
     size_t stride;        // bytes per CTA
     // byte offsets inside a CTA's slab
-    size_t oMasks;        // (MAXM + 2) * maxwords u32
+    size_t oMasks;        // (MAXM + 2) * maxwords u32 (slot SLOT_BEST doubles as a symbol-space mask in k_finish)
     size_t oTabs;         // MAXT + ENG_NW (staging) Tab
     size_t oHdrs;         // MAXH Hdr
     size_t oHists;        // (MAXM + 2) * 320 u32
     size_t oTabHash;      // MAXT u64
     size_t oDc;           // LCN * maxwords * 32 short: literal-cost arrays
-    size_t oKd;           // maxwords * 32 u16: per symbol, (length symbol - 256) | distance symbol << 5 (0: not a match)
-    size_t oMinfo;        // maxwords * 32 u32
+    size_t oMinfo;        // maxwords * 32 u32: per match, its packed record (build_views)
+    size_t oMout;         // maxwords * 32 u32: per match, the pool offset of its first decoded byte
+    size_t oMflag;        // maxwords u32: per symbol word, which of its symbols are matches
+    size_t oMrank;        // maxwords u32: per symbol word, the matches before its first symbol
+    size_t oLitHist;      // 320 u32: histogram of the block's literals and EOB
     size_t oTileFirst;    // maxtiles u32
     size_t oTrialAll;     // MAXT * 56 int
     size_t oRecs;         // 2 Cand: B and the winner
     size_t oSlowWs;       // ENG_NW TreeWs<290, 584>
-    size_t oPerm;         // maxwords * 32 u32: the block's matches grouped by length symbol
+    size_t oPerm;         // maxwords * 32 u32: the block's match ranks grouped by length symbol
     size_t oDcBits;       // DCN * 2 * maxwords u32: per cost array, the matches with a negative / a zero entry
     size_t oItems;        // maxwords + 64 u32: stretches of <= 32 entries of perm with one length symbol
     uint32_t maxwords, maxtiles;
 };
-// lays the slab out; returns the stride
+// lays the slab out; returns the stride.  maxwords bounds the symbol words of a block, so it bounds its match words too.
 inline size_t eng_scratch_layout(EngScratch& sc, uint32_t maxwords, uint64_t maxu) {
     sc.maxwords = maxwords;
     sc.maxtiles = (uint32_t)(maxu / DC_TILE + 4);
@@ -162,12 +169,15 @@ inline size_t eng_scratch_layout(EngScratch& sc, uint32_t maxwords, uint64_t max
     sc.oRecs = take(2 * sizeof(Cand));
     sc.oTabHash = take(sizeof(unsigned long long) * MAXT);
     sc.oTabs = take(sizeof(Tab) * (MAXT + ENG_NW));
+    sc.oLitHist = take(4 * 320);
+    sc.oMflag = take(4 * (size_t)maxwords);
+    sc.oMrank = take(4 * (size_t)maxwords);
     sc.oTileFirst = take(4 * (size_t)sc.maxtiles);
     sc.oMinfo = take(4 * maxn);
+    sc.oMout = take(4 * maxn);
     sc.oPerm = take(4 * maxn);
     sc.oItems = take(4 * ((size_t)maxwords + 64));
     sc.oDc = take(2 * maxn * LCN);
-    sc.oKd = take(2 * maxn);
     sc.oDcBits = take(4 * (size_t)maxwords * 2 * DCN);
     sc.oMasks = take(4 * (size_t)(MAXM + 2) * maxwords);
     sc.oHists = take(4 * (size_t)(MAXM + 2) * 320);
@@ -179,8 +189,8 @@ inline size_t eng_scratch_layout(EngScratch& sc, uint32_t maxwords, uint64_t max
 }
 
 struct Eng {
-    // cost-array values that are not costs: a match with a byte that has no code, a symbol that is not a match
-    static constexpr short DC_BLOCKED = 0x7FFF, DC_NOT_MATCH = 0x7FFE;
+    // cost-array value that is not a cost: a match with a byte that has no code
+    static constexpr short DC_BLOCKED = 0x7FFF;
     BlkView v;
     uint32_t* masks;
     uint32_t maxwords, maxn;
@@ -189,13 +199,16 @@ struct Eng {
     uint32_t* hists;
     unsigned long long* tabHash;
     short* dc;            // literal-cost arrays (LCN slots of maxn)
-    uint16_t* kd;         // per symbol: (length symbol - 256) | distance symbol << 5; 0 = not a match
-    uint32_t* minfo;
-    uint32_t* tileFirst;
+    uint32_t* minfo;      // per match: len-3 | dist symbol << 9 | (length symbol - 256) << 14 | (start in its cost tile) << 19
+    uint32_t* mout;       // per match: pool offset of its first decoded byte
+    uint32_t* mflag;      // per symbol word: bit b = symbol 32k + b is a match
+    uint32_t* mrank;      // per symbol word: rank of its first match
+    uint32_t* litHist;    // the block's literals and EOB: the part of every histogram that no pass changes
+    uint32_t* tileFirst;  // per cost tile: the first match that starts in it or later
     int* trialAll;
     Cand* recs;
     TreeWs<290, 584>* slowWs;
-    uint32_t* perm;       // symbol indices of the block's matches, grouped by length symbol (ES->binStart)
+    uint32_t* perm;       // ranks of the block's matches, grouped by length symbol (ES->binStart)
     uint32_t* dcBits;     // per cost array: maxwords words 'entry < 0', then maxwords words 'entry == 0'
     uint32_t* items;      // work items of the least-expensive statistics: first perm index | length symbol bin << 27
     int tid;
@@ -333,84 +346,152 @@ struct Eng {
     }
 
     // ---- block load -----------------------------------------------------------------------------------------------
-    // per-symbol views the passes read: kind (0 = not a match, else length symbol - 256) and
-    // minfo = len-3 | dist symbol << 9 | kind << 14 | (start offset in its cost tile) << 19 (0 for non-matches);
-    // tileFirst[t] = first symbol that starts in tile t.  Tiles count from the 16-byte boundary at or below the block's
-    // first decoded byte.
+    __device__ __forceinline__ uint32_t sym_words() const { return (v.n + 31) / 32; }
+
+    // The views the passes read, all indexed by match rank j: minfo[j] (see its declaration), mout[j], perm (the ranks
+    // grouped by length symbol) and tileFirst[t] = first match that starts in tile t or later (tiles count from the
+    // 16-byte boundary at or below the block's first decoded byte); mflag / mrank translate symbol words to ranks;
+    // litHist = the histogram of the literals and the EOB.  Sets v.nm and v.nwords.
     __device__ __noinline__ void build_views() {
-        const uint32_t a0 = (uint32_t)(v.out_off & ~15ull);
-        const uint32_t ntiles = (uint32_t)(((v.out_off - a0) + v.ulen) / DC_TILE) + 2;
+        const int lane = tid & 31, wid = tid >> 5;
+        const uint32_t nsw = sym_words();
 #pragma unroll 1
-        for (uint32_t t = tid; t < ntiles; t += ENG_NT) tileFirst[t] = v.n;
-        __syncthreads();
-#pragma unroll 1
-        for (uint32_t i = tid; i < v.n; i += ENG_NT) {
-            const uint32_t s = v.sym[i];
-            const uint32_t rel = v.symout[i] - a0;
-            const bool mt = sym_is_match(s);
-            const uint32_t kq = mt ? (uint32_t)(sym_lensym(s) - 256) : 0u;
-            const uint32_t dsy = mt ? (uint32_t)dist_sym(sym_dist(s)) : 0u;
-            minfo[i] = mt ? ((s & 0x1FF) | (dsy << 9) | (kq << 14) | ((rel & (DC_TILE - 1)) << 19)) : 0u;
-            kd[i] = (uint16_t)(kq | (dsy << 5));
-            const uint32_t ti = rel / DC_TILE;
-            const int tprev = i ? (int)((v.symout[i - 1] - a0) / DC_TILE) : -1;   // a symbol is shorter than a tile: ti - tprev <= 1
-            if ((int)ti != tprev) tileFirst[ti] = i;
+        for (uint32_t k = (uint32_t)wid; k < nsw; k += ENG_NW) {
+            const uint32_t i = 32 * k + (uint32_t)lane;
+            const uint32_t f = __ballot_sync(0xffffffffu, i < v.n && sym_is_match(v.sym[i]));
+            if (lane == 0) mflag[k] = f;
         }
-        // the matches grouped by length symbol (counting sort; the order inside a group does not matter)
+#pragma unroll 1
+        for (int k = tid; k < 320; k += ENG_NT) ES->hist[k] = 0;
         if (tid < 32) ES->leastCnt[tid] = 0;
         __syncthreads();
+        // ranks: every thread owns a contiguous run of symbol words, CTA-wide exclusive scan of their match counts
+        {
+            const uint32_t per = (nsw + ENG_NT - 1) / ENG_NT;
+            const uint32_t k0 = min(nsw, (uint32_t)tid * per), k1 = min(nsw, k0 + per);
+            uint32_t c = 0;
 #pragma unroll 1
-        for (uint32_t i = tid; i < v.n; i += ENG_NT) { const uint32_t s = v.sym[i]; if (sym_is_match(s)) atomicAdd(&ES->leastCnt[sym_lensym(s) - 257], 1); }
+            for (uint32_t k = k0; k < k1; k++) c += (uint32_t)__popc(mflag[k]);
+            uint32_t incl = c;
+#pragma unroll
+            for (int dd = 1; dd < 32; dd <<= 1) { const uint32_t y = __shfl_up_sync(0xffffffffu, incl, dd); if (lane >= dd) incl += y; }
+            if (lane == 31) ES->wt[wid] = incl;
+            __syncthreads();
+            uint32_t base = incl - c, total = 0;
+#pragma unroll 1
+            for (int w = 0; w < ENG_NW; w++) { const uint32_t x = ES->wt[w]; if (w < wid) base += x; total += x; }
+#pragma unroll 1
+            for (uint32_t k = k0; k < k1; k++) { mrank[k] = base; base += (uint32_t)__popc(mflag[k]); }
+            v.nm = total;
+            v.nwords = (total + 31) / 32;
+        }
         __syncthreads();
+        // match records; literals and EOB into the fixed histogram
+        const uint32_t a0 = (uint32_t)(v.out_off & ~15ull);
+#pragma unroll 1
+        for (uint32_t k = (uint32_t)wid; k < nsw; k += ENG_NW) {
+            const uint32_t i = 32 * k + (uint32_t)lane;
+            if (i >= v.n) continue;
+            const uint32_t f = mflag[k];
+            const uint32_t s = v.sym[i];
+            if ((f >> lane) & 1) {
+                const uint32_t j = mrank[k] + (uint32_t)__popc(f & ((1u << lane) - 1u));
+                const uint32_t so = v.symout[i];
+                const uint32_t kq = (uint32_t)(sym_lensym(s) - 256), dsy = (uint32_t)dist_sym(sym_dist(s));
+                minfo[j] = (s & 0x1FF) | (dsy << 9) | (kq << 14) | (((so - a0) & (DC_TILE - 1)) << 19);
+                mout[j] = so;
+                atomicAdd(&ES->leastCnt[kq - 1], 1);
+            } else if (s <= 256) atomicAdd(&ES->hist[s], 1u);
+        }
+        const uint32_t ntiles = (uint32_t)(((v.out_off - a0) + v.ulen) / DC_TILE) + 2;
+#pragma unroll 1
+        for (uint32_t t = tid; t < ntiles; t += ENG_NT) tileFirst[t] = v.nm;
+        __syncthreads();
+#pragma unroll 1
+        for (int k = tid; k < 320; k += ENG_NT) litHist[k] = ES->hist[k];
+        // tileFirst: match j fills the tiles after its predecessor's up to its own (tiles without a match start included)
+#pragma unroll 1
+        for (uint32_t j = tid; j < v.nm; j += ENG_NT) {
+            const uint32_t ti = (mout[j] - a0) / DC_TILE;
+            const uint32_t t0 = j ? (mout[j - 1] - a0) / DC_TILE + 1 : 0u;
+#pragma unroll 1
+            for (uint32_t t = t0; t <= ti; t++) tileFirst[t] = j;
+        }
+        // the matches grouped by length symbol (counting sort; the order inside a group does not matter)
         if (tid == 0) {
             uint32_t acc = 0;
 #pragma unroll 1
             for (int b = 0; b < 32; b++) { ES->binStart[b] = acc; acc += (uint32_t)ES->leastCnt[b]; ES->leastCnt[b] = (int)ES->binStart[b]; }
             ES->binStart[32] = acc;
-        }
-        __syncthreads();
-        if (tid == 0) {
-            uint32_t acc = 0;
+            acc = 0;
 #pragma unroll 1
             for (int b = 0; b < 32; b++) { ES->itemStart[b] = acc; acc += (ES->binStart[b + 1] - ES->binStart[b] + 31) / 32; }
             ES->itemStart[32] = acc;
         }
-#pragma unroll 1
-        for (uint32_t i = tid; i < v.n; i += ENG_NT) {
-            const uint32_t s = v.sym[i];
-            if (sym_is_match(s)) perm[atomicAdd(&ES->leastCnt[sym_lensym(s) - 257], 1)] = i;
-        }
         __syncthreads();
+#pragma unroll 1
+        for (uint32_t j = tid; j < v.nm; j += ENG_NT) perm[atomicAdd(&ES->leastCnt[((minfo[j] >> 14) & 31) - 1], 1)] = j;
         if (tid < 32) {
             uint32_t o = ES->itemStart[tid];
 #pragma unroll 1
             for (uint32_t j = ES->binStart[tid]; j < ES->binStart[tid + 1]; j += 32) items[o++] = j | ((uint32_t)tid << 27);
         }
-#pragma unroll 1
-        for (uint32_t i = v.n + tid; i < v.nwords * 32; i += ENG_NT) {
-            minfo[i] = 0; kd[i] = 0;
-        }
         __syncthreads();
     }
 
-    // histogram of the symbol list with mask `mid` into ES->hist, from the symbols
+    // symbol-space mask words src -> match-space mask in slot `slot` (bits on symbols that are not matches are dropped)
+    __device__ __noinline__ void load_mask(const uint32_t* src, int slot) {
+        uint32_t* md = maskp(slot);
+#pragma unroll 1
+        for (uint32_t k = tid; k < v.nwords; k += ENG_NT) md[k] = 0;
+        __syncthreads();
+#pragma unroll 1
+        for (uint32_t k = tid; k < sym_words(); k += ENG_NT) {
+            const uint32_t m = src[k];
+            uint32_t f = mflag[k];
+            if (!(m & f)) continue;
+            uint32_t x = 0;
+#pragma unroll 1
+            for (int c = 0; f; f &= f - 1, c++) x |= ((m >> (__ffs((int)f) - 1)) & 1u) << c;
+            const uint32_t r = mrank[k], sh = r & 31;
+            atomicOr(&md[r >> 5], x << sh);
+            if (sh && (x >> (32 - sh))) atomicOr(&md[(r >> 5) + 1], x >> (32 - sh));
+        }
+        __syncthreads();
+    }
+    // match-space mask in slot `slot` -> symbol-space mask words dst
+    __device__ __noinline__ void store_mask(int slot, uint32_t* dst) {
+        const uint32_t* ms = maskp(slot);
+#pragma unroll 1
+        for (uint32_t k = tid; k < sym_words(); k += ENG_NT) {
+            uint32_t f = mflag[k], out = 0;
+            if (f) {
+                const uint32_t r = mrank[k], sh = r & 31, w = r >> 5;
+                uint32_t x = ms[w] >> sh;
+                if (sh && w + 1 < v.nwords) x |= ms[w + 1] << (32 - sh);
+#pragma unroll 1
+                for (int c = 0; f; f &= f - 1, c++) out |= ((x >> c) & 1u) << (__ffs((int)f) - 1);
+            }
+            dst[k] = out;
+        }
+    }
+
+    // histogram of the symbol list with mask `mid` into ES->hist: the literal histogram plus the matches
     __device__ __noinline__ void pass_hist_full(int mid) {
         P0();
         const uint32_t* m = maskp(mid);
 #pragma unroll 1
-        for (int k = tid; k < 320; k += ENG_NT) ES->hist[k] = 0;
+        for (int k = tid; k < 320; k += ENG_NT) ES->hist[k] = litHist[k];
         __syncthreads();
 #pragma unroll 1
-        for (uint32_t i = tid; i < v.n; i += ENG_NT) {
-            uint32_t s = v.sym[i];
-            if (!sym_is_match(s)) {
-                if (s <= 256) atomicAdd(&ES->hist[s], 1u);
-            } else if (!((m[i >> 5] >> (i & 31)) & 1)) {
-                atomicAdd(&ES->hist[sym_lensym(s)], 1u);
-                atomicAdd(&ES->hist[288 + dist_sym(sym_dist(s))], 1u);
+        for (uint32_t j = tid; j < v.nm; j += ENG_NT) {
+            const uint32_t mi = minfo[j];
+            if (!((m[j >> 5] >> (j & 31)) & 1)) {
+                atomicAdd(&ES->hist[256 + ((mi >> 14) & 31)], 1u);
+                atomicAdd(&ES->hist[288 + ((mi >> 9) & 31)], 1u);
             } else {
-                const uint8_t* p = v.out + v.symout[i];
-                int len = sym_len(s);
+                const uint8_t* p = v.out + mout[j];
+                const int len = (int)(mi & 0x1FF) + 3;
 #pragma unroll 1
                 for (int k = 0; k < len; k++) atomicAdd(&ES->hist[p[k]], 1u);
             }
@@ -508,19 +589,17 @@ struct Eng {
         __syncthreads();
     }
 
-    // a new block: symbol view set by the caller, candidate `src` (global), mask words `maskSrc`
+    // a new block: symbol view set by the caller, candidate `src` (global), symbol-space mask words `maskSrc`
     __device__ __noinline__ void load_block(const Cand& src, const uint32_t* maskSrc, bool toFixed) {
         P0();
         __syncthreads();
         bigWeights = v.ulen + (uint64_t)v.n + 4 >= (1ull << 22);
-        uint32_t* mb = maskp(SLOT_B);
-#pragma unroll 1
-        for (uint32_t k = tid; k < v.nwords; k += ENG_NT) mb[k] = maskSrc[k];
         uint32_t* d = (uint32_t*)&recs[0];
         const uint32_t* s = (const uint32_t*)&src;
 #pragma unroll 1
         for (int k = tid; k < (int)(sizeof(Cand) / 4); k += ENG_NT) d[k] = s[k];
         build_views();
+        load_mask(maskSrc, SLOT_B);
         pass_hist_full(SLOT_B);
         uint32_t* hb = histp(SLOT_B);
 #pragma unroll 1
@@ -553,18 +632,18 @@ struct Eng {
         if (tid < 32) ES->refL[tid] = (uint8_t)(tb.L[256 + tid] + (tid > 0 && tid < 30 ? len_ebits_of(256 + tid) : 0));
         else if (tid < 64) ES->refD[tid - 32] = (uint8_t)(tb.D[tid - 32] + (tid - 32 < 30 ? dist_ebits_of(tid - 32) : 0));
     }
-    // cost-array entry of symbol i under the table whose refL / refD are loaded
-    __device__ __forceinline__ int dc_val(const short* lit, uint32_t i) const {
-        const int x = lit[i];
+    // cost-array entry of match j under the table whose refL / refD are loaded
+    __device__ __forceinline__ int dc_val(const short* lit, uint32_t j) const {
+        const int x = lit[j];
         if (x == DC_BLOCKED) return DC_BLOCKED;
-        const uint32_t k = kd[i];
-        return x - ES->refL[k & 31] - ES->refD[k >> 5];
+        const uint32_t mi = minfo[j];
+        return x - ES->refL[(mi >> 14) & 31] - ES->refD[(mi >> 9) & 31];
     }
 
     // the literal-cost array of table t's literal lengths.  ONE coalesced pass over the block's decoded bytes when it is
     // not cached: every warp streams its own run of 512-byte tiles (a 128-bit load per lane, code lengths looked up in
     // shared memory, a warp-wide prefix sum into its slice of shared memory) and every match that starts in a tile takes
-    // P[end] - P[start]; the one match that crosses the tile's end is finished from the next tile.
+    // P[end] - P[start]; the one match that crosses the tile's end is finished from the next tile.  Entry j = match j.
     __device__ __noinline__ const short* ensure_lit(int t) {
         int ls = ES->tabLit[t];
         if (ls == 0xFF) {   // which set of literal lengths is this?
@@ -632,8 +711,8 @@ struct Eng {
         const uint32_t ntiles = endRel / DC_TILE + 1;
         const uint32_t per = (ntiles + ENG_NW - 1) / ENG_NW;
         const uint32_t T0 = (uint32_t)wid * per, T1 = min(ntiles, T0 + per);
-        // Software pipeline, one tile deep: while tile T is processed, the bytes of T+1, the symbol range of T+2 and the
-        // first DC_PRE * 32 symbol records of T+1 are already in flight; the match that crosses from T into T+1 travels in
+        // Software pipeline, one tile deep: while tile T is processed, the bytes of T+1, the match range of T+2 and the
+        // first DC_PRE * 32 match records of T+1 are already in flight; the match that crosses from T into T+1 travels in
         // lane 0's registers.  P[k] holds the prefix of byte k relative to its lane's first byte, LB[l] the prefix of lane
         // l's first byte: the prefix at byte k is LB[k / 16] + P[k] (P[DC_TILE] = 0, LB[32] = tile total).
         constexpr int DC_PRE = 4;
@@ -641,7 +720,7 @@ struct Eng {
         int carryIdx = -1;
         uint32_t carryPart = 0, carryEnd = 0;
         uint4 q = make_uint4(0, 0, 0, 0);
-        uint32_t i0 = 0, i1 = 0, i2 = 0;       // symbols of the current tile: [i0, i1); of the next one: [i1, i2)
+        uint32_t i0 = 0, i1 = 0, i2 = 0;       // matches of the current tile: [i0, i1); of the next one: [i1, i2)
         uint32_t m0 = 0, m1 = 0, m2 = 0, m3 = 0;
         if (T0 < T1) {
             const uint32_t idx = T0 * DC_TILE + 16u * (uint32_t)lane;
@@ -654,7 +733,8 @@ struct Eng {
         }
         if (lane == 0) P[DC_TILE] = 0;
 #define D4_PFX(k) (LB[(k) >> 4] + P[(k)])
-        // one symbol record: a match inside the tile gets its literal cost, the one that crosses the tile's end is remembered
+        // one match record (0: none): a match inside the tile gets its literal cost, the one that crosses the tile's end is
+        // remembered
 #define D4_DC_ONE(i_, m_)                                                                                        \
         do {                                                                                                     \
             const uint32_t mm = (m_);                                                                            \
@@ -675,7 +755,7 @@ struct Eng {
             const uint4 cur = q;
             const uint32_t ci0 = i0, ci1 = i1;
             const uint32_t c0 = m0, c1 = m1, c2 = m2, c3 = m3;
-            if (T + 1 <= T1 && T + 1 <= ntiles) {   // next tile: its bytes, its first symbol records, the range after it
+            if (T + 1 <= T1 && T + 1 <= ntiles) {   // next tile: its bytes, its first match records, the range after it
                 const uint32_t nidx = idx + DC_TILE;
                 q = (nidx < endRel) ? *(const uint4*)(base + nidx) : make_uint4(0, 0, 0, 0);
                 i0 = ci1; i1 = i2;
@@ -730,7 +810,7 @@ struct Eng {
                 D4_DC_ONE(ib + 64, c2);
                 D4_DC_ONE(ib + 96, c3);
 #pragma unroll 1
-                for (uint32_t i = ib + 32u * DC_PRE; i < ci1; i += 32) { const uint32_t mx = minfo[i]; D4_DC_ONE(i, mx); }   // many short symbols
+                for (uint32_t i = ib + 32u * DC_PRE; i < ci1; i += 32) { const uint32_t mx = minfo[i]; D4_DC_ONE(i, mx); }   // many short matches
                 // hand the crossing match (if any) to lane 0
                 const unsigned who = __ballot_sync(0xffffffffu, nIdx >= 0);
                 if (who) {
@@ -749,9 +829,9 @@ struct Eng {
         return d;
     }
 
-    // the sign masks of table t's cost array: bit i of negW / zerW = entry i is negative / zero.  One streaming pass over
-    // the literal costs and the symbols' (length symbol, distance symbol) pairs, eight symbols (one mask byte) per thread
-    // and step.  Leaves refL / refD of t in shared memory.
+    // the sign masks of table t's cost array: bit j of negW / zerW = entry j is negative / zero.  One streaming pass over
+    // the literal costs and the match records, eight matches (one mask byte) per thread and step.  Leaves refL / refD of
+    // t in shared memory.
     __device__ __noinline__ const uint32_t* ensure_masks(int t, const short* lit) {
         load_ref(t);
         int slot = ES->tabDc[t];
@@ -772,51 +852,50 @@ struct Eng {
         uint32_t* negW = dcBits + (size_t)slot * 2 * maxwords;
         uint8_t* negB = (uint8_t*)negW;
         uint8_t* zerB = (uint8_t*)(negW + maxwords);
-        const uint32_t end = v.nwords * 32;
-        uint32_t i0 = (uint32_t)tid * 8;
-        uint4 lq = make_uint4(0, 0, 0, 0), kq = lq;
-        if (i0 < end) { kq = *(const uint4*)(kd + i0); lq = *(const uint4*)(lit + i0); }
+        const uint32_t end = v.nwords * 32, nm = v.nm;
+        uint32_t j0 = (uint32_t)tid * 8;
+        uint4 lq = make_uint4(0, 0, 0, 0), mq0 = lq, mq1 = lq;
+        if (j0 < nm) { lq = *(const uint4*)(lit + j0); mq0 = *(const uint4*)(minfo + j0); mq1 = *(const uint4*)(minfo + j0 + 4); }
 #pragma unroll 1
-        while (i0 < end) {
-            const uint4 cl = lq, ck = kq;
-            const uint32_t nx = i0 + ENG_NT * 8;
-            if (nx < end) { kq = *(const uint4*)(kd + nx); lq = *(const uint4*)(lit + nx); }
+        while (j0 < end) {
+            const uint4 cl = lq, c0 = mq0, c1 = mq1;
+            const uint32_t nx = j0 + ENG_NT * 8;
+            if (nx < nm) { lq = *(const uint4*)(lit + nx); mq0 = *(const uint4*)(minfo + nx); mq1 = *(const uint4*)(minfo + nx + 4); }
             uint32_t nb = 0, zb = 0;
-            if (ck.x | ck.y | ck.z | ck.w) {
-                const uint32_t lw[4] = {cl.x, cl.y, cl.z, cl.w}, kw[4] = {ck.x, ck.y, ck.z, ck.w};
+            if (j0 < nm) {
+                const uint32_t lw[4] = {cl.x, cl.y, cl.z, cl.w}, mw[8] = {c0.x, c0.y, c0.z, c0.w, c1.x, c1.y, c1.z, c1.w};
 #pragma unroll
                 for (int u = 0; u < 8; u++) {
-                    const uint32_t k = (u & 1) ? (kw[u >> 1] >> 16) : (kw[u >> 1] & 0xffffu);
                     const int x = (int)(short)((u & 1) ? (lw[u >> 1] >> 16) : (lw[u >> 1] & 0xffffu));
-                    if (k && x != DC_BLOCKED) {
-                        const int val = x - ES->refL[k & 31] - ES->refD[k >> 5];
+                    if (j0 + u < nm && x != DC_BLOCKED) {
+                        const int val = x - ES->refL[(mw[u] >> 14) & 31] - ES->refD[(mw[u] >> 9) & 31];
                         nb |= (val < 0 ? 1u : 0u) << u;
                         zb |= (val == 0 ? 1u : 0u) << u;
                     }
                 }
             }
-            negB[i0 >> 3] = (uint8_t)nb;
-            zerB[i0 >> 3] = (uint8_t)zb;
-            i0 = nx;
+            negB[j0 >> 3] = (uint8_t)nb;
+            zerB[j0 >> 3] = (uint8_t)zb;
+            j0 = nx;
         }
         __syncthreads();
         P1(PR_MASKS);
         return negW;
     }
 
-    // match i leaves the symbol list and its bytes enter it as literals: histogram delta in ES->hist
-    __device__ __noinline__ void hist_delta_replace(uint32_t i) {
-        const uint32_t s = v.sym[i];
-        atomicSub(&ES->hist[sym_lensym(s)], 1u);
-        atomicSub(&ES->hist[288 + dist_sym(sym_dist(s))], 1u);
-        const uint8_t* p = v.out + v.symout[i];
-        const int len = sym_len(s);
+    // match j leaves the symbol list and its bytes enter it as literals: histogram delta in ES->hist
+    __device__ __noinline__ void hist_delta_replace(uint32_t j) {
+        const uint32_t mi = minfo[j];
+        atomicSub(&ES->hist[256 + ((mi >> 14) & 31)], 1u);
+        atomicSub(&ES->hist[288 + ((mi >> 9) & 31)], 1u);
+        const uint8_t* p = v.out + mout[j];
+        const int len = (int)(mi & 0x1FF) + 3;
 #pragma unroll 1
         for (int k = 0; k < len; k++) atomicAdd(&ES->hist[p[k]], 1u);
     }
     // The same for every match a pass has just replaced, with the whole CTA: the pass queues the matches, then a thread
     // per short match (its bytes loaded eight at a time) and a warp per long one apply the delta.
-    // all 32 lanes call this together with the matches (bits of `nbits`, symbols i0 ..) each of them replaced in this step:
+    // all 32 lanes call this together with the matches (bits of `nbits`, ranks i0 ..) each of them replaced in this step:
     // one shared-memory atomic per warp and step instead of one per match
     __device__ __noinline__ void hq_push_warp(uint32_t nbits, uint32_t i0, int lane) {
         const uint32_t cnt = (uint32_t)__popc(nbits);
@@ -848,7 +927,7 @@ struct Eng {
         for (uint32_t j = tid; j < nS; j += ENG_NT) {
             const uint32_t i = ES->u.hq.qs[j];
             const uint32_t mi = minfo[i];
-            const uint32_t so = v.symout[i];
+            const uint32_t so = mout[i];
             if (lit) sv -= dc_val(lit, i);
             const int len = (int)(mi & 0x1FF) + 3;
             atomicSub(&ES->hist[256 + ((mi >> 14) & 31)], 1u);
@@ -879,7 +958,7 @@ struct Eng {
         for (uint32_t j = (uint32_t)(tid >> 5); j < nL; j += ENG_NW) {
             const uint32_t i = ES->u.hq.ql[j];
             const int len = (int)(minfo[i] & 0x1FF) + 3;
-            const uint8_t* p = v.out + v.symout[i];
+            const uint8_t* p = v.out + mout[i];
 #pragma unroll 1
             for (int k = lane; k < len; k += 32) atomicAdd(&ES->hist[p[k]], 1u);
         }
@@ -895,7 +974,7 @@ struct Eng {
 
     // replaceBackrefsWithLiteralsIfSmaller(prune) for memo slot `slot` = (mid, tabid): the candidates are the matches
     // whose cost-array entry is negative (prune: not positive) and that the mask does not cover yet - one AND of the
-    // cost array's sign words with the mask words, a word (32 symbols) per thread and step; the entries themselves are
+    // cost array's sign words with the mask words, a word (32 matches) per thread and step; the entries themselves are
     // only read for the (few) matches that are replaced.
     __device__ __noinline__ void pass_replace(int slot, int mid, int tabid, bool prune) {
         if (ES->sym.nMasks >= MAXM) { if (tid == 0) ES->sym.overflow = 1; __syncthreads(); return; }
@@ -984,14 +1063,14 @@ struct Eng {
 #pragma unroll
                     for (int u = 0; u < 8; u++) idx[u] = j + u < jend ? perm[j + u] : 0u;
 #pragma unroll
-                    for (int u = 0; u < 8; u++) { xv[u] = d[idx[u]]; mk[u] = mbytes[idx[u] >> 3] | ((uint32_t)kd[idx[u]] << 8); }
+                    for (int u = 0; u < 8; u++) { xv[u] = d[idx[u]]; mk[u] = mbytes[idx[u] >> 3] | (minfo[idx[u]] & (31u << 9)); }
 #pragma unroll
                     for (int u = 0; u < 8; u++) {
                         const bool live = j + u < jend && !((mk[u] >> (idx[u] & 7)) & 1);   // still a match
                         seen |= live;
                         const bool blk = live && xv[u] == DC_BLOCKED;
                         blocked |= blk;
-                        if (live && !blk) { sum += xv[u] - ES->refL[bin + 1] - ES->refD[mk[u] >> 13]; cnt++; }
+                        if (live && !blk) { sum += xv[u] - ES->refL[bin + 1] - ES->refD[mk[u] >> 9]; cnt++; }
                     }
                 }
                 if (seen) atomicOr(&ES->leastSeen, 1u << bin);
@@ -1778,8 +1857,11 @@ __device__ inline void eng_init(Eng& e, const EngScratch& sc, int cta) {
     e.hists = reinterpret_cast<uint32_t*>(base + sc.oHists);
     e.tabHash = reinterpret_cast<unsigned long long*>(base + sc.oTabHash);
     e.dc = reinterpret_cast<short*>(base + sc.oDc);
-    e.kd = reinterpret_cast<uint16_t*>(base + sc.oKd);
     e.minfo = reinterpret_cast<uint32_t*>(base + sc.oMinfo);
+    e.mout = reinterpret_cast<uint32_t*>(base + sc.oMout);
+    e.mflag = reinterpret_cast<uint32_t*>(base + sc.oMflag);
+    e.mrank = reinterpret_cast<uint32_t*>(base + sc.oMrank);
+    e.litHist = reinterpret_cast<uint32_t*>(base + sc.oLitHist);
     e.tileFirst = reinterpret_cast<uint32_t*>(base + sc.oTileFirst);
     e.trialAll = reinterpret_cast<int*>(base + sc.oTrialAll);
     e.recs = reinterpret_cast<Cand*>(base + sc.oRecs);

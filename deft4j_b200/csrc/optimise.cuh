@@ -82,7 +82,8 @@ __device__ inline void eng_view(Eng& e, const BlkState& b, const uint32_t* sym, 
     e.v.symout = symout + b.sym_off;
     e.v.out = out;
     e.v.n = n;
-    e.v.nwords = (n + 31) / 32;
+    e.v.nm = 0;       // (load_block counts the matches)
+    e.v.nwords = 0;
     e.v.ulen = ulen;
     e.v.out_off = b.out_off;
 }
@@ -150,9 +151,7 @@ k_opt_blocks(const uint32_t* __restrict__ jobs, uint32_t njobs, BlkState* __rest
             const uint32_t* s = (const uint32_t*)&e.recs[0];
             uint32_t* d = (uint32_t*)&b.cand;
             for (int k = tid; k < (int)(sizeof(Cand) / 4); k += ENG_NT) d[k] = s[k];
-            const uint32_t* m = e.maskp(SLOT_B);
-            uint32_t* pm = maskpool + b.mask_off;
-            for (uint32_t k = tid; k < e.v.nwords; k += ENG_NT) pm[k] = m[k];
+            e.store_mask(SLOT_B, maskpool + b.mask_off);
         }
         if (tid == 0) b.nrounds = r;
         __syncthreads();
@@ -327,8 +326,8 @@ __device__ void finish_stream(EngSmem& S, Eng& e, StreamState& st, BlkState* __r
                 // the merged mask is assembled in the pool region of A, which has room for the union (the regions of A, a
                 // removed block in between and B are adjacent); B's own region is left alone until the merge is accepted
                 {
-                    uint32_t* m = e.maskp(SLOT_BEST);   // scratch until the round materialises its winner
-                    for (uint32_t k = tid; k < e.v.nwords; k += ENG_NT) m[k] = 0;
+                    uint32_t* m = e.maskp(SLOT_BEST);   // symbol-space scratch until the round materialises its winner
+                    for (uint32_t k = tid; k < e.sym_words(); k += ENG_NT) m[k] = 0;
                     __syncthreads();
                     const uint32_t* ma = maskpool + c.mask_off;
                     const uint32_t* mb = maskpool + nx.mask_off;
@@ -355,9 +354,7 @@ __device__ void finish_stream(EngSmem& S, Eng& e, StreamState& st, BlkState* __r
                         const uint32_t* s = (const uint32_t*)&e.recs[1];
                         uint32_t* d = (uint32_t*)&c.cand;
                         for (int k = tid; k < (int)(sizeof(Cand) / 4); k += ENG_NT) d[k] = s[k];
-                        const uint32_t* bm = e.maskp(SLOT_BEST);
-                        uint32_t* pm = maskpool + c.mask_off;
-                        for (uint32_t k = tid; k < e.v.nwords; k += ENG_NT) pm[k] = bm[k];
+                        e.store_mask(SLOT_BEST, maskpool + c.mask_off);
                     }
                     __syncthreads();
                     if (tid == 0) {
