@@ -572,10 +572,25 @@ class Batch {
     }
 
     // per-CTA engine scratch: one contiguous, 2 MiB aligned slab per CTA (engine.cuh eng_scratch_layout)
+    // Every CTA gets a slab sized for the largest job, so one large stream among many small ones would ask for grid times
+    // its slab.  The kernels take their jobs from a counter, so `grid` is lowered to what the device can hold (free
+    // memory plus what the stream-ordered pool keeps in reserve, less a margin); fewer CTAs only take longer.
     unsigned char* scratch_raw = nullptr;
-    cudaError_t alloc_scratch(EngScratch& sc, unsigned grid, uint32_t maxwords, uint64_t maxu) {
+    cudaError_t alloc_scratch(EngScratch& sc, unsigned& grid, uint32_t maxwords, uint64_t maxu) {
         const size_t stride = eng_scratch_layout(sc, maxwords, maxu);
         const size_t align = (size_t)2 << 20;
+        size_t freeb = 0, totalb = 0;
+        if (cudaMemGetInfo(&freeb, &totalb) == cudaSuccess) {
+            cudaMemPool_t pool;
+            uint64_t res = 0, used = 0;
+            if (cudaDeviceGetDefaultMemPool(&pool, g_device) == cudaSuccess &&
+                cudaMemPoolGetAttribute(pool, cudaMemPoolAttrReservedMemCurrent, &res) == cudaSuccess &&
+                cudaMemPoolGetAttribute(pool, cudaMemPoolAttrUsedMemCurrent, &used) == cudaSuccess && res > used)
+                freeb += (size_t)(res - used);
+            const size_t margin = ((size_t)1 << 30) + totalb / 16;
+            const size_t fit = freeb > margin + align ? (freeb - margin - align) / stride : 0;
+            grid = (unsigned)std::max<size_t>(1, std::min<size_t>(grid, fit));
+        }
         cudaError_t e = dalloc(&scratch_raw, stride * grid + align, cs);
         if (e != cudaSuccess) return e;
         sc.slab = (unsigned char*)(((uintptr_t)scratch_raw + align - 1) & ~(uintptr_t)(align - 1));
@@ -663,7 +678,7 @@ class Batch {
             cudaFuncSetAttribute(k_finish, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
             D4_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_finish, ENG_NT, 0));
             if (perSM < 1) perSM = 1;
-            const unsigned grid = (unsigned)std::min<uint64_t>(n, (uint64_t)g_sms * perSM);
+            unsigned grid = (unsigned)std::min<uint64_t>(n, (uint64_t)g_sms * perSM);
             unsigned* d_counter = nullptr;
             D4_CUDA_CHECK(dalloc(&d_counter, 1, cs));
             D4_CUDA_CHECK(cudaMemsetAsync(d_counter, 0, 4, cs));

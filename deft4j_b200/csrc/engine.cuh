@@ -60,14 +60,32 @@ struct BlkView {
 };
 
 constexpr int DC_TILE = 512;      // decoded bytes per cost-array tile: one 16-byte load per lane of a warp
-constexpr int DCN = 16;           // per-table sign masks kept per block (round-robin eviction)
-constexpr int LCN = 12;           // literal-cost arrays kept per block (round-robin eviction)
-constexpr int MAXLIT = 64;        // distinct sets of literal code lengths tracked per block
-constexpr int WS_BYTES = 3072;    // per-warp workspace for trees / header work
+// Cache and queue capacities.  Each is a macro so that a stress build can shrink it until every eviction, reset and
+// overflow path runs on ordinary inputs (__graft_entry__.build: libdeft4cu_stress.so); the product build uses the defaults.
+#ifndef D4_DCN
+#define D4_DCN 16
+#endif
+#ifndef D4_LCN
+#define D4_LCN 12
+#endif
+#ifndef D4_MAXLIT
+#define D4_MAXLIT 64
+#endif
 #ifndef D4_HQS
 #define D4_HQS 4608
 #endif
-constexpr int HQS = D4_HQS, HQL = 1024;   // queue of freshly replaced matches (all / long ones) for the histogram update
+#ifndef D4_HQL
+#define D4_HQL 1024
+#endif
+constexpr int DCN = D4_DCN;       // per-table sign masks kept per block (round-robin eviction)
+constexpr int LCN = D4_LCN;       // literal-cost arrays kept per block (round-robin eviction)
+constexpr int MAXLIT = D4_MAXLIT; // distinct sets of literal code lengths tracked per block
+constexpr int WS_BYTES = 3072;    // per-warp workspace for trees / header work
+constexpr int HQS = D4_HQS, HQL = D4_HQL;   // queue of freshly replaced matches (all / long ones) for the histogram update
+// a pass holds one literal-cost array and one sign-mask slot at a time; the slot indices are stored in unsigned chars
+// whose 0xFF means "none"
+static_assert(DCN >= 1 && DCN < 0xFF && LCN >= 1 && LCN < 0xFF && MAXLIT >= 1 && MAXLIT < 0xFF, "cache sizes");
+static_assert(HQS >= 1 && HQL >= 1, "queue sizes");
 constexpr int SLOT_B = MAXM, SLOT_BEST = MAXM + 1;   // extra mask / histogram slots: the records of B and of the winner
 static_assert(DC_TILE == 32 * 16 && DC_TILE > 258, "a tile is one warp-wide 128-bit load and no match spans more than two tiles");
 
@@ -594,6 +612,9 @@ struct Eng {
         P0();
         __syncthreads();
         bigWeights = v.ulen + (uint64_t)v.n + 4 >= (1ull << 22);
+#ifdef D4_FORCE_BIG_WEIGHTS   // stress build: every tree takes the slow, exact-weight path
+        bigWeights = true;
+#endif
         uint32_t* d = (uint32_t*)&recs[0];
         const uint32_t* s = (const uint32_t*)&src;
 #pragma unroll 1
