@@ -5,7 +5,7 @@ libdeft4cu.so (include/deft4cu.h).  All deflate work runs in hand-written CUDA k
 there is no CPU fallback.
 """
 from .deflate_stream import DeflateStream
-from .deft import Deft, optimise_batch
+from .deft import Deft, compress_batch, optimise_batch
 from . import container
 
-__all__ = ["DeflateStream", "Deft", "optimise_batch", "container"]
+__all__ = ["DeflateStream", "Deft", "compress_batch", "optimise_batch", "container"]

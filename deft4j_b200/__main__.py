@@ -1,4 +1,4 @@
-"""`python -m deft4j_b200 optimise|optimise-folder ...` — mirror of deft4j-cmd (SURVEY.md §8f row 4).
+"""`python -m deft4j_b200 optimise|optimise-folder|gzip-compress ...` — mirror of deft4j-cmd (SURVEY.md §8f row 4).
 
 cmd/Main.java:8-25 (subcommands), cmd/Optimise.java:15-54, cmd/OptimiseFolder.java:33-67 and
 cmd/CMDUtil.java:57-181: same positional arguments, option names, stdout/stderr lines, temp-file overwrite protocol
@@ -209,6 +209,32 @@ def optimise_files_batched(paths, merge_blocks, stream_cls, out, err, max_bytes=
     return ok
 
 
+def gzip_compress_file(inp, outp, merge_blocks, block_bytes, stream_cls, out=None, err=None):
+    """`gzip-compress`: the input's bytes compressed and optimised on the device, wrapped in a gzip member with GZFile's
+    default header."""
+    from .container.gz_file import GZFile
+    out, err = out or sys.stdout, err or sys.stderr
+    if not os.path.isfile(inp):
+        print("Error: Input file does not exist", file=err)
+        return False
+    if os.path.isdir(outp):
+        print("Error: Output file is a directory", file=err)
+        return False
+    with open(inp, "rb") as f:
+        data = f.read()
+    stream = stream_cls.compress_batch([data], block_bytes=block_bytes)[0]
+    if stream is None:
+        print("Failed to compress input file", file=err)
+        return False
+    saved = stream.optimise(merge_blocks)
+    if saved != 0:
+        print("Saved %d bits with optimisation" % saved, file=out)
+    gz = GZFile(stream_cls)
+    gz.setData(stream)
+    _write_back(outp, gz.write(), inp, err)
+    return True
+
+
 def main(argv=None, out=None, err=None, stream_cls=None):
     """`stream_cls` lets a caller supply another implementation of the DeflateStream interface (the CPU-only tests
     pass their checker); the command line always uses the CUDA engine."""
@@ -233,8 +259,23 @@ def main(argv=None, out=None, err=None, stream_cls=None):
     p = sub.add_parser("optimise-folder", help="Optimise every recognised file below a folder, in place")
     p.add_argument("inputFolder")
     common(p)
+    p = sub.add_parser("gzip-compress", help="Compress a file to gzip with this library's own device compressor",
+                       description="Compress inputFile into a gzip file on the GPU: LZ77 matching and a lazy parse into "
+                       "fixed-coded blocks, then this optimiser's block rewriting.  The compressor is this library's own; "
+                       "its bytes are not those of the reference's gzip-compress, whose compressors are not available here.")
+    p.add_argument("inputFile", help="The file to compress")
+    p.add_argument("outputFile", help="The gzip file to write")
+    p.add_argument("--merge-blocks", "-b", dest="merge_blocks", action="store_true", default=False,
+                   help="Also try merging deflate blocks (off by default: on large stationary inputs it is slow)")
+    p.add_argument("--block-bytes", type=int, default=0,
+                   help="Input bytes per deflate block, 256..65535 (default 32768)")
     a = ap.parse_args(argv)
     cls = stream_cls or _stream_cls()
+    if a.cmd == "gzip-compress":
+        ok = gzip_compress_file(a.inputFile, a.outputFile, a.merge_blocks, a.block_bytes, cls, out, err)
+        if not ok:
+            print("Failed to compress " + a.inputFile, file=err)
+        return 0 if ok else 1
     if a.cmd == "optimise":
         try:
             ok = optimise_file(a.inputFile, a.outputFile, a.format, a.raw, a.merge_blocks, cls, out, err)

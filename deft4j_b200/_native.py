@@ -44,9 +44,11 @@ SYMBOLS = {
     "deft4cu_last_error": (C.c_char_p, []),
     "deft4cu_version": (C.c_char_p, []),
     "deft4cu_optimise_batch": (C.c_int, [_U8PP, _U64P, C.c_uint32, C.c_uint32, C.POINTER(Result)]),
+    "deft4cu_compress_batch": (C.c_int, [_U8PP, _U64P, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Result)]),
     "deft4cu_free_results": (None, [C.POINTER(Result), C.c_uint32]),
     "deft4cu_stream_parse": (C.c_int, [C.c_char_p, C.c_uint64, _PP, _U64P]),
     "deft4cu_stream_parse_batch": (C.c_int, [_U8PP, _U64P, C.c_uint32, _PP, C.POINTER(C.c_int32), _U64P]),
+    "deft4cu_stream_compress_batch": (C.c_int, [_U8PP, _U64P, C.c_uint32, C.c_uint32, _PP, C.POINTER(C.c_int32)]),
     "deft4cu_stream_free": (None, [_P]),
     "deft4cu_stream_optimise": (C.c_int, [_P, C.c_uint32, C.POINTER(C.c_int64)]),
     "deft4cu_stream_optimise_batch": (C.c_int, [_PP, C.c_uint32, C.c_uint32, C.POINTER(C.c_int64)]),

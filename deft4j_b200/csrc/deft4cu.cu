@@ -21,6 +21,7 @@ static void set_error(const std::string& s) { g_err = s; }
 
 #include "write.cuh"
 #include "checksum.cuh"
+#include "lzcomp.cuh"
 
 namespace d4 {
 
@@ -205,6 +206,8 @@ class Batch {
     bool parsed = false;
     bool optimised = false;
     bool too_big = false;   // parse() refused: the decoded size of the batch does not fit the 32-bit pools (split it)
+    bool compressed = false;   // the model was built by compress() from raw bytes (the input must never be parsed)
+    uint32_t block_bytes = 0;  // compress(): input bytes per block
 
     ~Batch() { release_all(); if (own_cs) cudaStreamDestroy(own_cs); }
 
@@ -213,7 +216,7 @@ class Batch {
         dfree(d_sym, cs); dfree(d_symout, cs); dfree(d_out, cs);
         dfree(d_blk_stream, cs); dfree(d_bs, cs); dfree(d_logs, cs); dfree(d_maskpool, cs);
         dfree(d_sstate, cs); dfree(d_gerr, cs); dfree(d_dst, cs); dfree(d_dst_off, cs);
-        parsed = false; have_sums = false; optimised = false;
+        parsed = false; compressed = false; have_sums = false; optimised = false;
     }
     void release_all() {
         HostTimer ht("release");
@@ -532,7 +535,23 @@ class Batch {
             for (uint32_t c = chain_off[i]; c < chain_off[i + 1]; c++)
                 if (winfos[chain[c]].status != ST_OK && infos[i].status == ST_OK) infos[i].status = ST_PARSE;
         dfree(d_summ, cs); dfree(d_jobs, cs); dfree(d_chunks, cs);
-        // model
+        {
+            const int rc = init_model(sblk_base);
+            if (rc) return rc;
+        }
+        float t;
+        cudaEventElapsedTime(&t, ev[0], ev[1]); ms[0] = t;
+        cudaEventElapsedTime(&t, ev[1], ev[2]); ms[1] = t;
+        cudaEventElapsedTime(&t, ev[2], ev[3]); ms[2] = t;
+        ms[7] = (float)parse_rewalks;  // walkers whose guessed start was wrong or missing
+        for (auto& e : ev) cudaEventDestroy(e);
+        parsed = true;
+        return DEFT4CU_OK;
+    }
+
+    // the optimiser's model of a batch whose blocks, symbols and decoded bytes are in place (parse() and compress()):
+    // mask offsets, per-stream state and the BlkState of every block
+    int init_model(const std::vector<uint64_t>& sblk_base) {
         mask_offs.resize(nblk_total);
         uint64_t mo = 0;
         for (uint64_t b = 0; b < nblk_total; b++) { mask_offs[b] = mo; mo += (summ[b].n_sym + 31) / 32; }
@@ -556,18 +575,134 @@ class Batch {
         D4_CUDA_CHECK(dalloc(&d_maskpool, mo + 2, cs));
         D4_CUDA_CHECK(dalloc(&d_sstate, n, cs));
         D4_CUDA_CHECK(cudaMemsetAsync(d_maskpool, 0, (mo + 2) * 4, cs));
+        // the stream states go to the device now as well: a handle may be written before it is optimised
+        D4_CUDA_CHECK(cudaMemcpyAsync(d_sstate, sstate.data(), sizeof(StreamState) * n, cudaMemcpyHostToDevice, cs));
         D4_CUDA_CHECK(cudaMemcpyAsync(d_moffs, mask_offs.data(), 8 * nblk_total, cudaMemcpyHostToDevice, cs));
         D4_CUDA_CHECK(cudaMemcpyAsync(d_blk_stream, blk_stream.data(), 4 * nblk_total, cudaMemcpyHostToDevice, cs));
         if (nblk_total) LAUNCH(k_init_state, (unsigned)((nblk_total + 127) / 128), 128, cs, d_blocks, d_moffs, d_bs, nblk_total);
         D4_CUDA_CHECK(cudaStreamSynchronize(cs));
         dfree(d_moffs, cs);
+        return DEFT4CU_OK;
+    }
+
+    // ---- compress: raw input bytes -> the model of their fixed-coded stream (lzrule.cuh, lzcomp.cuh) ----------------
+    int compress(uint32_t bytes_per_block) {
+        HostTimer ht("compress");
+        release_model();
+        too_big = false;
+        block_bytes = bytes_per_block;
+        cudaEvent_t ev[3];
+        for (auto& e : ev) cudaEventCreate(&e);
+        descs.assign(n + 1, StreamDesc{});
+        infos.assign(n, StreamInfo{});
+        D4_CUDA_CHECK(dalloc(&d_gerr, 8, cs));
+        D4_CUDA_CHECK(cudaMemsetAsync(d_gerr, 0, 8 * sizeof(int), cs));
+        // decoded bytes: the input itself, packed the way parse() packs them
+        uint64_t ob = 0;
+        for (uint32_t i = 0; i < n; i++) {
+            descs[i].out_base = ob;
+            infos[i].status = in_len[i] > 0xF0000000ull ? ST_UNSUPPORTED : ST_OK;
+            if (infos[i].status == ST_OK) ob += in_len[i];
+        }
+        descs[n].out_base = ob;
+        nout_total = ob;
+        uint64_t ob_max = 0xF8000000ull;   // decoded offsets are 32-bit
+        if (const char* e = getenv("D4_MAX_DECODED")) ob_max = std::min<uint64_t>(ob_max, strtoull(e, nullptr, 10));   // tests force the split
+        if (ob >= ob_max) {
+            too_big = true;
+            for (uint32_t i = 0; i < n; i++) if (infos[i].status == ST_OK) infos[i].status = ST_UNSUPPORTED;
+            set_error("decoded size of the batch exceeds 4 GiB; split the batch");
+            return DEFT4CU_ERR_UNSUPPORTED;
+        }
+        D4_CUDA_CHECK(dalloc(&d_out, ob + 16, cs));
+        for (uint32_t i = 0; i < n; i++)
+            if (infos[i].status == ST_OK && in_len[i])
+                D4_CUDA_CHECK(cudaMemcpyAsync(d_out + descs[i].out_base, d_in + in_off[i], in_len[i], cudaMemcpyDeviceToDevice, cs));
+        // blocks of `bytes_per_block` input bytes, the last one shorter; an empty stream is one block holding only EOB
+        std::vector<LzJob> jobs;
+        std::vector<uint64_t> sblk_base(n);
+        blk_stream.clear();
+        for (uint32_t i = 0; i < n; i++) {
+            sblk_base[i] = jobs.size();
+            if (infos[i].status != ST_OK) continue;
+            const uint64_t len = in_len[i], nb = len ? (len + bytes_per_block - 1) / bytes_per_block : 1;
+            for (uint64_t k = 0; k < nb; k++) {
+                LzJob jb{};
+                jb.base = descs[i].out_base; jb.n = len;
+                jb.s = (uint32_t)(k * bytes_per_block); jb.e = (uint32_t)std::min<uint64_t>(len, (k + 1) * bytes_per_block);
+                jb.bfinal = k + 1 == nb;
+                jobs.push_back(jb);
+                blk_stream.push_back(i);
+            }
+        }
+        nblk_total = jobs.size();
+        LzJob* d_jobs = nullptr;
+        LzRes* d_res = nullptr;
+        uint32_t* d_m = nullptr;
+        uint2* d_ent = nullptr;
+        uint16_t* d_slab = nullptr;
+        unsigned* d_counter = nullptr;
+        D4_CUDA_CHECK(dalloc(&d_jobs, nblk_total, cs));
+        D4_CUDA_CHECK(dalloc(&d_res, nblk_total, cs));
+        D4_CUDA_CHECK(dalloc(&d_m, ob + 1, cs));
+        D4_CUDA_CHECK(dalloc(&d_ent, nblk_total * LZ_NT, cs));
+        D4_CUDA_CHECK(dalloc(&d_counter, 1, cs));
+        D4_CUDA_CHECK(cudaMemsetAsync(d_counter, 0, 4, cs));
+        D4_CUDA_CHECK(cudaMemcpyAsync(d_jobs, jobs.data(), sizeof(LzJob) * nblk_total, cudaMemcpyHostToDevice, cs));
+        int perSM = 0;
+        D4_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&perSM, k_lz_match, LZ_NT, LZ_SMEM));
+        const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>(nblk_total, (uint64_t)g_sms * std::max(perSM, 1)));
+        D4_CUDA_CHECK(dalloc(&d_slab, (size_t)grid * LZ_WIN_CAP, cs));
+        cudaEventRecord(ev[0], cs);
+        if (nblk_total) LAUNCH_SM(k_lz_match, grid, LZ_NT, LZ_SMEM, cs, d_jobs, (uint32_t)nblk_total, d_out, d_m, d_slab, d_ent, d_res, d_counter);
+        cudaEventRecord(ev[1], cs);
+        std::vector<LzRes> lres(nblk_total);
+        D4_CUDA_CHECK(cudaMemcpyAsync(lres.data(), d_res, sizeof(LzRes) * nblk_total, cudaMemcpyDeviceToHost, cs));
+        D4_CUDA_CHECK(cudaStreamSynchronize(cs));
+        if (stage && cs == own_cs) { host_release(stage); stage = nullptr; }   // upload()'s copy is behind us
+        dfree(d_slab, cs); dfree(d_counter, cs);
+        // symbol pool bases and block positions: exclusive scans over the batch and over each stream
+        uint64_t sb = 0;
+        summ.resize(nblk_total);
+        for (uint32_t i = 0; i < n; i++) {
+            descs[i].sym_base = sb;
+            StreamInfo& si = infos[i];
+            if (si.status != ST_OK) continue;
+            uint64_t bit = 0;
+            const uint64_t nb = (i + 1 < n ? sblk_base[i + 1] : nblk_total) - sblk_base[i];
+            for (uint64_t k = sblk_base[i]; k < sblk_base[i] + nb; k++) {
+                jobs[k].sym_base = sb; jobs[k].hdr_bit = bit;
+                sb += lres[k].n_sym;
+                bit += 3 + lres[k].payload;
+                summ[k] = BlkSummary{1u, lres[k].n_sym, jobs[k].e - jobs[k].s, 1u, 0u};
+                si.n_syms += lres[k].n_sym;
+            }
+            si.n_blocks = (uint32_t)nb;
+            si.out_len = in_len[i];
+            si.consumed = in_len[i];
+            si.total_bits = si.end_bit = bit;
+            si.final_seen = 1;
+        }
+        descs[n].sym_base = sb;
+        nsym_total = sb;
+        D4_CUDA_CHECK(cudaMemcpyAsync(d_jobs, jobs.data(), sizeof(LzJob) * nblk_total, cudaMemcpyHostToDevice, cs));
+        D4_CUDA_CHECK(dalloc(&d_sym, sb, cs));
+        D4_CUDA_CHECK(dalloc(&d_symout, sb, cs));
+        D4_CUDA_CHECK(dalloc(&d_blocks, nblk_total, cs));
+        if (nblk_total) LAUNCH(k_lz_emit, (unsigned)nblk_total, LZ_NT, cs, d_jobs, d_out, d_m, d_ent, d_res, d_sym, d_symout, d_blocks);
+        cudaEventRecord(ev[2], cs);
+        dfree(d_jobs, cs); dfree(d_res, cs); dfree(d_m, cs); dfree(d_ent, cs);
+        {
+            const int rc = init_model(sblk_base);
+            if (rc) return rc;
+        }
         float t;
-        cudaEventElapsedTime(&t, ev[0], ev[1]); ms[0] = t;
-        cudaEventElapsedTime(&t, ev[1], ev[2]); ms[1] = t;
-        cudaEventElapsedTime(&t, ev[2], ev[3]); ms[2] = t;
-        ms[7] = (float)parse_rewalks;  // walkers whose guessed start was wrong or missing
+        cudaEventElapsedTime(&t, ev[0], ev[1]); ms[0] = t;   // match + parse
+        cudaEventElapsedTime(&t, ev[1], ev[2]); ms[1] = t;   // emit (and the host scan between them)
+        ms[2] = 0; ms[7] = 0;
         for (auto& e : ev) cudaEventDestroy(e);
         parsed = true;
+        compressed = true;
         return DEFT4CU_OK;
     }
 
@@ -835,6 +970,7 @@ int deft4cu_init(int device) {
     D4_CUDA_CHECK(cudaGetDeviceProperties(&p, device));
     g_sms = p.multiProcessorCount;
     D4_CUDA_CHECK(cudaFuncSetAttribute(k_count, cudaFuncAttributeMaxDynamicSharedMemorySize, WIN_BYTES + WIN_SLACK + 16));
+    D4_CUDA_CHECK(cudaFuncSetAttribute(k_lz_match, cudaFuncAttributeMaxDynamicSharedMemorySize, LZ_SMEM));
     cudaMemPool_t pool;
     if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
         uint64_t thr = ~0ull;
@@ -921,6 +1057,33 @@ int deft4cu_stream_parse_batch(const uint8_t* const* data, const uint64_t* len, 
     }
     return DEFT4CU_OK;
 }
+static int compress_block_bytes(uint32_t* block_bytes) {
+    if (*block_bytes == 0) *block_bytes = LZ_BLOCK_DEFAULT;
+    if (*block_bytes < LZ_BLOCK_MIN || *block_bytes > LZ_BLOCK_MAX) {
+        set_error("block_bytes must be 0 (default) or within [256, 65535]");
+        return DEFT4CU_ERR_ARG;
+    }
+    return DEFT4CU_OK;
+}
+int deft4cu_stream_compress_batch(const uint8_t* const* data, const uint64_t* len, uint32_t n, uint32_t block_bytes,
+                                  deft4cu_stream** handles, int32_t* status) {
+    int rc = compress_block_bytes(&block_bytes);
+    if (rc) return rc;
+    rc = ensure_init();
+    if (rc) return rc;
+    auto b = std::make_shared<Batch>();
+    rc = b->upload(data, len, n);
+    if (rc) return rc;
+    rc = b->compress(block_bytes);
+    if (rc && rc != DEFT4CU_ERR_UNSUPPORTED) return rc;
+    for (uint32_t i = 0; i < n; i++) {
+        const int st = b->infos[i].status;
+        if (status) status[i] = st;
+        handles[i] = nullptr;
+        if (st == ST_OK) handles[i] = new deft4cu_stream{b, i};
+    }
+    return DEFT4CU_OK;
+}
 int deft4cu_stream_parse(const uint8_t* data, uint64_t len, deft4cu_stream** out, uint64_t* consumed) {
     int32_t st = 0;
     uint64_t c = 0;
@@ -944,8 +1107,12 @@ int deft4cu_stream_optimise_batch(deft4cu_stream* const* s, uint32_t n, uint32_t
     // usually arrives as one batch per stream.  Streams that have not been optimised yet are regrouped into ONE batch
     // (device-to-device copy of their input, parsed again together): one launch of every kernel for the whole list.
     if (batches.size() > 1) {
+        // A compressed batch's input is raw data: batches are regrouped only when all of them were parsed, or all of them
+        // were compressed with the same block size (and then compressed again together)
         bool fresh = true;
-        for (Batch* b : batches) fresh = fresh && !b->optimised && b->parsed;
+        for (Batch* b : batches)
+            fresh = fresh && !b->optimised && b->parsed && b->compressed == batches[0]->compressed &&
+                    b->block_bytes == batches[0]->block_bytes;
         for (uint32_t i = 0; i < n && fresh; i++)
             for (uint32_t k = 0; k < i; k++) if (s[k] == s[i]) fresh = false;   // a handle listed twice
         if (fresh) {
@@ -953,7 +1120,7 @@ int deft4cu_stream_optimise_batch(deft4cu_stream* const* s, uint32_t n, uint32_t
             for (uint32_t i = 0; i < n; i++) src[i] = {s[i]->batch.get(), s[i]->idx};
             auto nb = std::make_shared<Batch>();
             int rc = nb->upload_from(src);
-            if (rc == DEFT4CU_OK) rc = nb->parse();
+            if (rc == DEFT4CU_OK) rc = batches[0]->compressed ? nb->compress(batches[0]->block_bytes) : nb->parse();
             bool same = rc == DEFT4CU_OK;
             for (uint32_t i = 0; i < n && same; i++) same = nb->infos[i].status == ST_OK;
             if (same) {
@@ -1158,6 +1325,41 @@ int deft4cu_optimise_batch(const uint8_t* const* in, const uint64_t* in_len, uin
         const int r1 = deft4cu_optimise_batch(in, in_len, h, flags, results);
         if (r1 && r1 != DEFT4CU_ERR_UNSUPPORTED) return r1;
         const int r2 = deft4cu_optimise_batch(in + h, in_len + h, n - h, flags, results + h);
+        return r2 ? r2 : r1;
+    }
+    if (rc) {
+        if (rc == DEFT4CU_ERR_UNSUPPORTED && b.infos.size() == n) {
+            for (uint32_t i = 0; i < n; i++) { memset(&results[i], 0, sizeof results[i]); results[i].status = b.infos[i].status; }
+        }
+        return rc;
+    }
+    std::vector<uint8_t> sel(n, 1);
+    rc = b.optimise(flags, sel);
+    if (rc && rc != DEFT4CU_ERR_UNSUPPORTED) return rc;
+    int rc2 = b.write();
+    if (rc2) return rc2;
+    rc2 = b.checksums();
+    if (rc2) return rc2;
+    rc2 = fill_results(b, results, true);
+    return rc2 ? rc2 : rc;
+}
+int deft4cu_compress_batch(const uint8_t* const* in, const uint64_t* in_len, uint32_t n, uint32_t flags, uint32_t block_bytes,
+                           deft4cu_result* results) {
+    int rc = compress_block_bytes(&block_bytes);
+    if (rc) return rc;
+    rc = ensure_init();
+    if (rc) return rc;
+    Batch b;
+    rc = b.upload(in, in_len, n);
+    if (rc) return rc;
+    rc = b.compress(block_bytes);
+    if (rc == DEFT4CU_ERR_UNSUPPORTED && b.too_big && n > 1) {
+        // more than 4 GiB of input: the list is compressed in two halves (streams never interact)
+        b.release_all();
+        const uint32_t h = n / 2;
+        const int r1 = deft4cu_compress_batch(in, in_len, h, flags, block_bytes, results);
+        if (r1 && r1 != DEFT4CU_ERR_UNSUPPORTED) return r1;
+        const int r2 = deft4cu_compress_batch(in + h, in_len + h, n - h, flags, block_bytes, results + h);
         return r2 ? r2 : r1;
     }
     if (rc) {

@@ -476,3 +476,85 @@ void host_engine_best(void* p, uint8_t* L, uint8_t* D, int32_t* meta, int32_t* p
 }
 
 }  // extern "C"
+
+// =====================================================================================================================
+// The compressor's parse rule (lzrule.cuh) on the host: the fixed-coded stream F the device compressor models, written
+// with a plain serial hash chain over the whole stream.  The GPU's F is compared with this byte for byte.
+// =====================================================================================================================
+#include "lzrule.cuh"
+
+namespace {
+struct HostBits {
+    std::vector<uint8_t> out;
+    uint64_t acc = 0;
+    int n = 0;
+    void bits(uint32_t v, int c) {
+        acc |= (uint64_t)v << n;
+        n += c;
+        while (n >= 8) { out.push_back((uint8_t)acc); acc >>= 8; n -= 8; }
+    }
+    void code(uint32_t c, int len) {   // Huffman codes go MSB first
+        uint32_t r = 0;
+        for (int k = 0; k < len; k++) r |= ((c >> k) & 1u) << (len - 1 - k);
+        bits(r, len);
+    }
+    void fixed_lit(int s) {
+        if (s <= 143) code(0x30 + s, 8);
+        else if (s <= 255) code(0x190 + s - 144, 9);
+        else if (s <= 279) code(s - 256, 7);
+        else code(0xC0 + s - 280, 8);
+    }
+};
+struct HostByte { const uint8_t* d; __host__ __device__ uint8_t operator()(int64_t i) const { return d[i]; } };
+struct HostLink { const int64_t* prev; __host__ __device__ int64_t operator()(int64_t q) const { return prev[q]; } };
+}  // namespace
+
+extern "C" {
+
+// F for `n` bytes at block size `block`; returns its size in bits (-1: `cap` too small), bytes in out[0, ceil(bits / 8))
+long long host_lz_compress(const uint8_t* d, uint64_t n, uint32_t block, uint8_t* out, uint64_t cap) {
+    std::vector<int64_t> prev(n, -1), head(LZ_HASH_MASK + 1, -1);
+    for (uint64_t p = 0; p + 3 <= n; p++) {
+        const uint32_t h = lz_hash(d[p], d[p + 1], d[p + 2]);
+        prev[p] = head[h];
+        head[h] = (int64_t)p;
+    }
+    const HostByte byte{d};
+    const HostLink link{prev.data()};
+    HostBits w;
+    long long bits = 0;
+    const uint64_t nblk = n == 0 ? 1 : (n + block - 1) / block;
+    for (uint64_t b = 0; b < nblk; b++) {
+        const int64_t s = (int64_t)(b * block), e = (int64_t)std::min<uint64_t>(n, (b + 1) * block);
+        w.bits(b + 1 == nblk ? 1 : 0, 1);
+        w.bits(1, 2);
+        bits += 3;
+        std::vector<uint32_t> M(e - s + 1, 0);
+        for (int64_t p = s; p < e; p++) M[p - s] = lz_best_match(p, e, (int64_t)n, byte, link);
+        for (int64_t i = s; i < e;) {
+            const uint32_t m = lz_take(M[i - s], M[i + 1 - s], i + 1 == e);
+            if (m) {
+                const int len = (int)lz_mlen(m), dist = (int)lz_mdist(m);
+                const int ls = lz_len_sym(len), ds = dist_sym(dist);
+                w.fixed_lit(ls);
+                w.bits((uint32_t)(len - c_len_base[ls - 257]), len_ebits_of(ls));
+                w.code((uint32_t)ds, 5);
+                w.bits((uint32_t)(dist - c_dist_base[ds]), dist_ebits_of(ds));
+                bits += lz_fixed_match_bits(len, dist);
+                i += len;
+            } else {
+                w.fixed_lit(d[i]);
+                bits += lz_fixed_lit_bits(d[i]);
+                i++;
+            }
+        }
+        w.fixed_lit(256);
+        bits += LZ_FIXED_EOB_BITS;
+    }
+    if (w.n) w.bits(0, 8 - w.n);
+    if (w.out.size() > cap) return -1;
+    memcpy(out, w.out.data(), w.out.size());
+    return bits;
+}
+
+}  // extern "C"

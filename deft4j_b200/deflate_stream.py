@@ -74,6 +74,29 @@ class DeflateStream:
                 out.append(None)
         return out
 
+    @classmethod
+    def compress_batch(cls, buffers, names=None, block_bytes=0):
+        """Compress raw data buffers on the device (deft4cu_stream_compress_batch); returns a list of DeflateStream (None
+        where a buffer was refused) whose model is the fixed-coded stream of the data, ready for optimise."""
+        L = N.lib()
+        n = len(buffers)
+        ptrs, lens = N.make_ptr_arrays(buffers)
+        handles = (C.c_void_p * max(n, 1))()
+        status = (C.c_int32 * max(n, 1))()
+        rc = L.deft4cu_stream_compress_batch(ptrs, lens, n, block_bytes, handles, status)
+        if rc != N.OK:
+            raise N.Deft4cuError(N.last_error())
+        out = []
+        for i in range(n):
+            if status[i] == N.OK and handles[i]:
+                s = cls(names[i] if names else None)
+                s._h = C.c_void_p(handles[i])
+                s.consumed = len(buffers[i])
+                out.append(s)
+            else:
+                out.append(None)
+        return out
+
     # -- optimise(boolean mergeBlocks) (:496-566) -------------------------------------------------
     def optimise(self, mergeBlocks=True):
         return self.optimise_batch([self], mergeBlocks)[0]

@@ -36,6 +36,21 @@ def optimise_batch(buffers, mergeBlocks=True):
     ptrs, lens = N.make_ptr_arrays(buffers)
     res = (N.Result * max(n, 1))()
     rc = L.deft4cu_optimise_batch(ptrs, lens, n, N.MERGE_BLOCKS if mergeBlocks else 0, res)
+    return _results(L, rc, res, n)
+
+
+def compress_batch(buffers, mergeBlocks=True, block_bytes=0):
+    """Compression entry (deft4cu_compress_batch): list of raw data buffers -> list of dict results like optimise_batch's,
+    whose "out" is a raw deflate stream of the data.  block_bytes = 0 is the default block size (32768)."""
+    L = N.lib()
+    n = len(buffers)
+    ptrs, lens = N.make_ptr_arrays(buffers)
+    res = (N.Result * max(n, 1))()
+    rc = L.deft4cu_compress_batch(ptrs, lens, n, N.MERGE_BLOCKS if mergeBlocks else 0, block_bytes, res)
+    return _results(L, rc, res, n)
+
+
+def _results(L, rc, res, n):
     if rc in (N.ERR_CUDA, N.ERR_ARG):
         raise N.Deft4cuError(N.last_error())
     out = []

@@ -63,6 +63,16 @@ int  deft4cu_optimise_batch(const uint8_t* const* in, const uint64_t* in_len, ui
 void deft4cu_free_results(deft4cu_result* results, uint32_t n);
 
 /* ------------------------------------------------------------------------------------------------
+ * Compression — raw bytes in, optimised deflate out.  The device cuts every input into blocks of block_bytes
+ * (0: 32768; otherwise 256..65535, else DEFT4CU_ERR_ARG), finds LZ77 matches with a lazy parse and models the
+ * result as a fixed-coded stream F (the rule: deft4j_b200/csrc/lzrule.cuh), which the optimiser then entropy-codes.
+ * size_bits_in = bits of F, saved_bits = what optimise saved against F, consumed_bytes = uncompressed_len = input
+ * length.  flags honours DEFT4CU_MERGE_BLOCKS.  The output is this library's own; it is not any CPU compressor's.
+ * ---------------------------------------------------------------------------------------------- */
+int  deft4cu_compress_batch(const uint8_t* const* in, const uint64_t* in_len, uint32_t n, uint32_t flags,
+                            uint32_t block_bytes, deft4cu_result* results);
+
+/* ------------------------------------------------------------------------------------------------
  * Handle API — mirrors the DeflateStream object (base/deflate/DeflateStream.java)
  * ---------------------------------------------------------------------------------------------- */
 typedef struct deft4cu_stream deft4cu_stream;
@@ -72,6 +82,10 @@ int      deft4cu_stream_parse(const uint8_t* data, uint64_t len, deft4cu_stream*
 /* several streams parsed together (one launch); handles[i] is NULL where status[i] != OK */
 int      deft4cu_stream_parse_batch(const uint8_t* const* data, const uint64_t* len, uint32_t n,
                                     deft4cu_stream** handles, int32_t* status, uint64_t* consumed);
+/* handles of raw inputs compressed on the device (deft4cu_compress_batch's first step); writing one before optimise
+ * gives the fixed-coded stream F.  handles[i] is NULL where status[i] != OK. */
+int      deft4cu_stream_compress_batch(const uint8_t* const* data, const uint64_t* len, uint32_t n, uint32_t block_bytes,
+                                       deft4cu_stream** handles, int32_t* status);
 void     deft4cu_stream_free(deft4cu_stream* s);
 /* DeflateStream.optimise(boolean) (:496-566) */
 int      deft4cu_stream_optimise(deft4cu_stream* s, uint32_t flags, int64_t* saved_bits);
