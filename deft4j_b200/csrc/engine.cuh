@@ -1,7 +1,7 @@
 // engine.cuh — the block candidate engine: executes what the symbolic enumerator (enum.cuh) asks for.
 //
-// One CTA owns one block.  Thread 0 sweeps the enumeration of DeflateStream.optimiseBlock (DeflateStream.java:343-490)
-// over memo tables in shared memory; every miss becomes a request.  After a sweep the whole CTA computes the requests:
+// One CTA owns one block.  Lane 0 of every warp sweeps items of the enumeration of DeflateStream.optimiseBlock
+// (DeflateStream.java:343-490) over memo tables in shared memory; every miss becomes a request.  After a sweep the whole CTA computes the requests:
 //   passes   replaceBackrefsWithLiteralsIfSmaller / removeDistLitLeastExpensive (DeflateBlockHuffman.java:222-319,
 //            373-458): CTA-wide, 8 matches per thread, against a per-table cost array dc[j] = literal cost - match cost.
 //            The cost array of a table is built in ONE coalesced pass over the block's decoded bytes: 2 KiB tiles, per-byte
@@ -90,7 +90,7 @@ constexpr int SLOT_B = MAXM, SLOT_BEST = MAXM + 1;   // extra mask / histogram s
 static_assert(DC_TILE == 32 * 16 && DC_TILE > 258, "a tile is one warp-wide 128-bit load and no match spans more than two tiles");
 
 // cycle accounting per engine phase (-DD4_PROF builds only; read back with deft4cu_debug_prof): thread 0's clock64
-// deltas, [cat] = cycles, [32 + cat] = calls
+// deltas (a sweep counts up to the barrier after it, so it is the slowest sweeper's time), [cat] = cycles, [32 + cat] = calls
 #ifdef D4_PROF
 __device__ unsigned long long g_prof[64];
 #define P0() const long long p0_ = clock64()
@@ -107,8 +107,7 @@ enum { PR_BLOCK = 0, PR_ROUND, PR_SWEEP, PR_SELECT, PR_PASS, PR_DC, PR_RECODE, P
 
 struct EngSmem {
     SymState sym;
-    Enumer en;            // the selection sweep (thread 0) and the first discovery sweeper
-    Enumer enx[3];        // the other discovery sweepers (one seed of the enumeration each)
+    Enumer en;            // the block, the round's selection state, and the sweeper of a traced selection sweep
     TraceSink tsink;
     unsigned long long maskHash[MAXM];
     uint32_t hist[320];          // pass histogram delta / block histogram; [0,19) header pair frequencies
@@ -123,8 +122,7 @@ struct EngSmem {
     long long recPay[ENG_NW];
     uint32_t wt[ENG_NW];
     int redAny, redAny2, tmpIdx, err;
-    int sweepOk[4], segImproved, segmentedRound;
-    struct { long long bestSize, restMin; SC best; unsigned bestIndex, candIndex; int bestStored, bestArg; } carry;   // selection state carried into a sweep
+    int itemNext, segImproved, segmentedRound;   // itemNext: the next item of the current sweep
     unsigned char tabDc[MAXT];   // tabid -> sign-mask slot (0xFF: none)
     unsigned short dcOwner[DCN]; // slot -> tabid (0xFFFF: free)
     int dcNext;
@@ -141,6 +139,7 @@ struct EngSmem {
         unsigned char ws[ENG_NW][WS_BYTES];
         uint32_t P[ENG_NW][DC_TILE + 4 + 36]; // cost-array build: per warp, packed (cost | uncodable count << 16) prefixes of one tile + lane bases
         struct { Tab tab; Hdr hdr; TreeWsCL ws; } mat;   // winner materialisation (thread 0)
+        struct { Enumer w[ENG_NW]; ItemRec rec[NITEMS]; } sw;   // sweeps: the sweepers' enumerators, the selection of every item
         struct { uint32_t nS, nL; uint32_t qs[HQS]; uint32_t ql[HQL]; } hq;   // passes: matches that were just replaced
     } u;
 };
@@ -1695,76 +1694,48 @@ struct Eng {
     // sweeps + execution until the part `seg` of the enumeration is resolved, then the selection sweep.  Returns false on
     // a pool overflow (nothing selected).
     __device__ __noinline__ bool run_segment(unsigned seg) {
-        if (tid == 0) { ES->sym.doneMulti = 0; ES->sym.doneRun = 0; ES->sym.doneAor = 0; }
+        if (tid == 0) { ES->sym.doneItem = 0; ES->sym.doneAor = 0; ES->itemNext = 0; }
         __syncthreads();
-        constexpr int NSW = ENG_NW < 4 ? ENG_NW : 4;   // sweepers: lane 0 of the first warps, one seed (or two) each
-        // The last turn of the loop is the selection sweep.  The candidates of a seed form one contiguous stretch of the
-        // enumeration, so the sweepers select inside their own stretch (indices from 0, best so far = the value carried
-        // in) and thread 0 joins the stretches in order: first strict minimum, indices shifted by what came before.
-        // With the trace armed the candidates must come out in order: thread 0 sweeps alone.
+        // Lane 0 of every warp takes items (enum.cuh sweep_item) from a counter, each with its own copy of the enumerator.  The last
+        // turn of the loop is the selection sweep: every item selects inside its own candidates (indices from 0, best so
+        // far = the value carried in) into its record, and thread 0 joins the records in item order.  With the trace
+        // armed the candidates must come out in order: thread 0 sweeps every item alone.
         bool selecting = false;
         const bool par = ES->en.trace == nullptr;
 #pragma unroll 1
         for (int it = 0;; it++) {
-            const int t = tid >> 5;
-            if (selecting && par && tid == 0) {
-                ES->carry.bestSize = ES->en.bestSize; ES->carry.restMin = ES->en.restMin; ES->carry.best = ES->en.best;
-                ES->carry.bestIndex = ES->en.bestIndex; ES->carry.candIndex = ES->en.candIndex; ES->carry.bestStored = ES->en.bestStored;
-                ES->carry.bestArg = ES->en.bestArg;
-            }
-            if (selecting) __syncthreads();
-            if ((tid & 31) == 0 && t < NSW && (!selecting || par || t == 0)) {   // the one call site of the (inlined) sweep
-                P0();
-                Enumer& en = t == 0 ? ES->en : ES->enx[t - 1];
-                if (t) { en.B = ES->en.B; en.blockType = ES->en.blockType; en.storedOK = ES->en.storedOK; en.storedSize = ES->en.storedSize; en.trace = nullptr; en.trialAll = nullptr; en.internalError = 0; }
-                const bool whole = selecting && !par;
-                unsigned sg = seg;
-                if (selecting && par) {
-                    en.bestSize = ES->carry.bestSize; en.restMin = 0x7fffffffffffffffll; en.candIndex = 0; en.bestIndex = 0xffffffffu;
-                    en.bestStored = 0; en.bestArg = -1;
-                    if (t) sg &= ~(unsigned)Enumer::SEG_HEAD;
+            P0();   // a sweep is timed from here to the barrier after it: the slowest sweeper, and the join
+            const bool serial = selecting && !par;
+            const unsigned before = ES->en.bestIndex;
+            if ((tid & 31) == 0 && (!serial || tid == 0)) {
+                Enumer& en = serial ? ES->en : ES->u.sw.w[tid >> 5];
+                if (!serial) { en = ES->en; en.trace = nullptr; }
+                const long long carried = ES->en.bestSize;
+                int next = 0;
+#pragma unroll 1
+                while (true) {
+                    const int item = serial ? next++ : atomicAdd(&ES->itemNext, 1);
+                    if (item >= NITEMS) break;
+                    if (selecting && !serial) en.begin_item(carried);
+                    const bool ok = en.sweep_one(ES->sym, selecting, seg, item);   // the one call site of the (inlined) sweep
+                    if (selecting) {
+                        if (!ok || en.internalError) ES->err = ERR_INTERNAL;
+                        if (!serial) en.put_item(ES->u.sw.rec[item]);
+                    }
                 }
-                const unsigned before = ES->en.bestIndex;
-                const bool ok = en.sweep(ES->sym, selecting, sg, whole ? 0 : t * 4 / NSW, whole ? 4 : (t + 1) * 4 / NSW);
-                ES->sweepOk[t] = ok && !en.internalError ? 1 : 0;
-                if (selecting) {
-                    if (!par) ES->segImproved = ES->en.bestIndex != before && !ES->en.bestStored;
-                    if (en.internalError || en.poisoned) ES->err = ERR_INTERNAL;
-                    P1(PR_SELECT);
-                } else { P1(PR_SWEEP); }
             }
             __syncthreads();
+            if (tid == 0) ES->itemNext = 0;   // read again only after the barriers of collect_requests
             if (selecting) {
-                if (par) {
-                    if (tid == 0) {
-                        long long bs = ES->carry.bestSize, rm = ES->carry.restMin;
-                        unsigned bi = ES->carry.bestIndex, base = ES->carry.candIndex;
-                        int st = ES->carry.bestStored, arg = ES->carry.bestArg;
-                        SC best = ES->carry.best;
-                        bool improved = false;
-#pragma unroll 1
-                        for (int k = 0; k < NSW; k++) {
-                            const Enumer& e = k == 0 ? ES->en : ES->enx[k - 1];
-                            if (e.bestIndex != 0xffffffffu && e.bestSize < bs) {
-                                bs = e.bestSize; bi = base + e.bestIndex; st = e.bestStored; arg = e.bestArg; best = e.best;
-                                improved = !e.bestStored;
-                            }
-                            if (e.restMin < rm) rm = e.restMin;
-                            base += e.candIndex;
-                        }
-                        ES->en.bestSize = bs; ES->en.restMin = rm; ES->en.bestIndex = bi; ES->en.candIndex = base;
-                        ES->en.bestStored = st; ES->en.bestArg = arg; ES->en.best = best;
-                        ES->segImproved = improved ? 1 : 0;
-                    }
-                    __syncthreads();
-                }
+                if (tid == 0) ES->segImproved = par ? (ES->en.join(ES->u.sw.rec) ? 1 : 0) : (ES->en.bestIndex != before && !ES->en.bestStored);
+                __syncthreads();
+                P1(PR_SELECT);
                 return true;
             }
+            P1(PR_SWEEP);
             if (ES->sym.overflow) return false;
             collect_requests();
-            bool done = true;
-#pragma unroll 1
-            for (int k = 0; k < NSW; k++) done = done && ES->sweepOk[k];
+            const bool done = ES->sym.doneItem == (1u << NITEMS) - 1;
             const bool nothing = ES->sym.nqPass + ES->sym.nqRec + ES->sym.nqHdr + ES->sym.nqTrial == 0;
             if (done && nothing) { selecting = true; continue; }
             if (nothing || it > 4096) { if (tid == 0) ES->err = ERR_INTERNAL; __syncthreads(); return false; }

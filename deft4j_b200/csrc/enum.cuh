@@ -12,13 +12,15 @@
 //     recodeToFixedHuffman     mid -> payload                                     :637-653
 //     header mutators          (hid, op) -> hid'                                  :471-476,579-635
 //     56 header strategy trials  tabid -> (first-minimum bits, its index)         DeflateStream.java:277-316
-// ONE thread walks the reference's enumeration (multi -> run -> aor -> trials, the tie-break contract of SURVEY.md §8a)
-// over memo tables of those functions.  A miss whose inputs are known is queued as a request and poisons everything
-// that depends on it; after the sweep the whole CTA computes the queued requests side by side (engine.cuh: Huffman
-// trees of different requests in different warps, passes CTA-wide, header trials 28 threads per table) and the sweep
-// is repeated, skipping the sub-trees (aor / run / multi nodes) that completed earlier.  The enumeration does not depend
-// on which candidate is winning, so when a sweep raises no request a final sweep feeds every candidate to the selection
-// callback (DeflateStream.java:349-368) in the reference's order, with the reference's strict `<`.
+// The reference's enumeration (multi -> run -> aor -> trials, the tie-break contract of SURVEY.md §8a) is walked over
+// memo tables of those functions, cut into 17 items (the head and every (seed, variant)) that the lanes of a CTA
+// take from a queue.  A miss whose inputs are known is queued as a request and poisons everything that depends on it;
+// after the sweep the whole CTA computes the queued requests side by side (engine.cuh: Huffman trees of different
+// requests in different warps, passes CTA-wide, header trials 28 threads per table) and the sweep is repeated, skipping
+// the items that completed earlier.  The enumeration does not depend on which candidate is winning, so when a sweep
+// raises no request a final sweep feeds every candidate to the selection callback (DeflateStream.java:349-368) with the
+// reference's strict `<`: each item selects inside its own candidates and a join stitches the items back in the
+// reference's order.
 //
 // The file compiles as host code too (D4_HOST_TEST): tests/test_host_units.py drives this very enumerator with a plain
 // serial executor (hosttest.cu) against the oracle's candidate trace.
@@ -88,8 +90,8 @@ struct SymState {
     int nP;                            // used pass memo slots
     int nMasks, nTabs, nHdrs;
     int overflow;                      // a pool filled up during this round
-    unsigned doneMulti, doneRun;       // sub-trees that completed in an earlier sweep of this round
-    unsigned long long doneAor;
+    unsigned doneItem;                 // items (Enumer::sweep_item) that completed in an earlier sweep of this round
+    unsigned long long doneAor;        // ... and the bases (seed, variant, base) inside them
     int requested;                     // a sweep marked something PENDING since this was last cleared
 };
 
@@ -101,7 +103,7 @@ D4_HD void sym_reset(SymState& S, int tid, int nthreads) {
     if (tid == 0) {
         S.nqPass = S.nqRec = S.nqHdr = S.nqTrial = 0;
         S.nP = 0; S.nMasks = 0; S.nTabs = 0; S.nHdrs = 0; S.overflow = 0;
-        S.doneMulti = 0; S.doneRun = 0; S.doneAor = 0; S.requested = 0;
+        S.doneItem = 0; S.doneAor = 0; S.requested = 0;
     }
 }
 
@@ -136,6 +138,19 @@ struct TraceSink {
     unsigned* n;
 };
 
+// items of one sweep (Enumer::sweep_item): the head, then (seed, variant, base) in the reference's order
+constexpr int NITEMS = 1 + 4 * 4;
+static_assert(NITEMS <= 32, "one done bit per item");
+
+// selection outcome of one item swept apart (Enumer::put_item / join)
+struct ItemRec {
+    long long bestSize, restMin, sizeC1;
+    SC best;
+    unsigned bestIndex;    // inside the item's own candidates (0xffffffff: none beat the value carried in)
+    unsigned candIndex;    // candidates the item counted
+    int bestStored, bestArg;
+};
+
 struct Enumer {
     const int* trialAll;       // [tabid * 56 + k] header bits of every strategy (trace only; may be null)
     TraceSink* trace;          // null: no trace
@@ -154,7 +169,7 @@ struct Enumer {
     unsigned candIndex, bestIndex;
     SC best;
 
-    // Everything below is inlined into ONE routine (sweep, a single copy) without calls (the sweep runs in a single thread next to CTAs that
+    // Everything below is inlined into ONE routine (sweep_item, a single copy) without calls (the sweep runs in a single thread next to CTAs that
     // stream through L1: a call stack in local memory would cost an L2 round trip per access).  `st` is the block's
     // memo state (shared memory on the device).
 
@@ -293,116 +308,153 @@ struct Enumer {
         candIndex = 0; bestIndex = 0xffffffffu;
         best = B;
         internalError = 0;
-        st.doneMulti = 0; st.doneRun = 0; st.doneAor = 0;
+        st.doneItem = 0; st.doneAor = 0;
     }
 
-    // DeflateStream.optimiseBlock (:343-490) over the parts `seg` (the seeds mlo <= m < mhi: in discovery sweeps several
-    // threads take one seed each).  Returns true when the sweep met no missing or pending op.  The nesting is the reference's: runOptimisationsCallbackMulti (:443-463) over four seeds,
-    // runOptimisationsCallback (:400-442) over up to four variants of a seed, addOptimisedRecoded (:265-317) over three
-    // bases of a variant.
-    D4_HD bool sweep(SymState& st, bool sel, unsigned seg, int mlo = 0, int mhi = 4) {
-        SC wO, wH, wE, wX, wY, wB0, wB1, wB2, wB3, wPP;
+    // DeflateStream.optimiseBlock (:343-490) is cut into NITEMS items that can be swept in any order and by several
+    // threads at once.  The nesting is the reference's: runOptimisationsCallbackMulti (:443-463) over four seeds m,
+    // runOptimisationsCallback (:400-442) over up to four variants r of a seed, addOptimisedRecoded (:265-317) over three
+    // bases a of a variant.  Item 0 is the head (the optimised block and the stored candidate); item 1 + m * 4 + r is one
+    // variant of one seed with its three bases, and the items in index order emit the reference's candidates in its order.
+    // An item recomputes its prefix (the seed and the variant) through the memo tables; when the prefix is not known yet
+    // the item is poisoned and asks for nothing beyond what the prefix asked for, so a sweep over all items raises exactly
+    // the requests of one walk over the whole enumeration, whatever the order of the items.  Returns true when the item
+    // met no missing or pending op (an item outside `seg`, or an r = 3 variant that recodedHuffmanFull left unchanged, is
+    // empty and returns true).
+    D4_HD bool sweep_item(SymState& st, bool sel, unsigned seg, int item) {
         select = sel;
         poisoned = false;
-        if (sel && (seg & SEG_HEAD)) trace_put(-1, size(st, B));
+        const int m = (item - 1) >> 2, r = (item - 1) & 3;
         long long saved = 0;
-        wO = op_optimise(st, B, &saved);
-        bool hasO = wO.ok && saved > 0;
-        if (!wO.ok) poisoned = true;
-        if (seg & SEG_HEAD) {
+        SC wO = B, wH = B;
+        bool hasO = false;
+        if (item == 0 || (m == 1 && blockType != 1)) { wO = op_optimise(st, B, &saved); hasO = wO.ok && saved > 0; }
+        if (item == 0 && (seg & SEG_HEAD)) {
+            if (sel) trace_put(-1, size(st, B));
             if (hasO) { cb(st, wO, false); if (sel) sizeC1 = size(st, wO); }
             if (storedOK && sel) {
                 if (storedSize >= 0 && storedSize < bestSize) { bestSize = storedSize; bestStored = 1; bestIndex = candIndex; }
                 candIndex++;
             }
         }
-        wH = B;
-        bool hasOh = hasO;
-        if (blockType == 1) {
+        if (blockType == 1) {   // a FIXED block is recoded first; multi(O) starts from the recode's optimised form
             wH = op_recode(st, B);
-            wO = op_optimise(st, wH, &saved);
-            hasOh = wO.ok && saved > 0;
-            if (!wO.ok) poisoned = true;
+            if (item == 0 || m == 1) { wO = op_optimise(st, wH, &saved); hasO = wO.ok && saved > 0; }
         }
-        for (int m = mlo; m < mhi; m++) {
-            // ---- the seed of this runOptimisationsCallbackMulti ----------------------------------------------------
-            if (m == 0) { if (!(seg & SEG_MULTI_H)) continue; wE = wH; }
-            else if (m == 1) { if (!(seg & SEG_MULTI_O) || !hasOh) continue; wE = wO; }
-            else if (m == 2) {
-                if ((seg & SEG_FIXED) && blockType != 1) {   // the fixed-code candidate sits between multi(O) and the least seeds
-                    long long s2 = 0;
-                    const SC E = op_optimise(st, op_to_fixed(st, wH), &s2);
-                    cb(st, E);
-                }
-                if (!(seg & SEG_LEAST0)) continue;
-                wE = op_pass(st, wH, OP_LEAST0);
-            } else { if (!(seg & SEG_LEAST1)) continue; wE = op_pass(st, wH, OP_LEAST1); }
-            if (!select && ((st.doneMulti >> m) & 1)) continue;
-            const bool outerM = poisoned;
-            poisoned = false;
-            wX = wE;
-            for (int r = 0; r < 4; r++) {
-                // ---- the variant this runOptimisationsCallback works on ---------------------------------------------
-                if (r == 1) wX = op_recode(st, wE);
-                else if (r == 2) wX = op_recode_less(st, wE);
-                else if (r == 3) {
-                    bool full = false;
-                    wX = recoded_full(st, wX, &full);
-                    if (!wX.ok) { poisoned = true; break; }
-                    if (!full) break;
-                }
-                cb(st, wX);
-                const int rn = m * 4 + r;
-                if (!select && ((st.doneRun >> rn) & 1)) continue;
-                const bool outerR = poisoned;
-                poisoned = false;
-                for (int a = 0; a < 3; a++) {
-                    if (a == 0) {
-                        wY = op_hdr(st, wX, HOP_RECODE); cb(st, wY);                                  // post
-                        long long sv = 0;
-                        const SC o = op_optimise(st, wY, &sv); cb_if_saved(st, o, sv);             // post optimised
-                    } else wY = op_pass(st, wX, a == 1 ? OP_LEAST0 : OP_LEAST1);
-                    // ---- addOptimisedRecoded(y) ---------------------------------------------------------------------
-                    const int an = rn * 3 + a;
-                    int nb = 0;
-                    if (select || !((st.doneAor >> an) & 1)) {
-                        const bool outerA = poisoned;
-                        poisoned = false;
-                        // the four bases are only ever read by the trials: their Tab and payload.  Every trial rewrites the
-                        // header from the Tab (optimiseBlockDynBlock -> rewriteHeader, DeflateStream.java:184-198), so the
-                        // header half of DeflateBlockHuffman.optimise() cannot influence any candidate here and is not run.
-                        wB0 = op_pass(st, wY, OP_REPLACE);                                  // optimiseBlockCopyHelper(toOptimise)
-                        wB1 = op_pass(st, op_recode(st, wY), OP_REPLACE);                   // optimiseBlockHelper(recodedHuffman(.., false))
-                        wPP = op_recode_less(st, wY);                                       // pruned
-                        wB2 = op_pass(st, wPP, OP_REPLACE);                                 // optimiseBlockCopyHelper(pruned)
-                        bool full = false;
-                        wB3 = recoded_full(st, wPP, &full);                                       // prunedFull
-                        if (wB3.ok) {
-                            nb = full ? 4 : 3;
-                            if (full) wB3 = op_pass(st, wB3, OP_REPLACE);
-                            trial_base(st, wB0); trial_base(st, wB1); trial_base(st, wB2);
-                            if (full) trial_base(st, wB3);
-                        } else poisoned = true;
-                        if (!poisoned) D4_OR_U64(&st.doneAor, 1ull << an);
-                        poisoned = poisoned || outerA;
-                    }
-                    if (a == 0) {
-                        const SC t = op_hdr(st, wX, HOP_RECODE_LESS); cb(st, t);                    // pruned header
-                        long long sv = 0;
-                        const SC o = op_optimise(st, t, &sv); cb_if_saved(st, o, sv);
-                        // addOptimisedRecoded(prune) (:431) re-evaluates candidates with exactly the sizes of the sweep on `post`
-                        // (both are copies of the same block that differ only in the header, which every base / trial
-                        // discards), so under the strict `<` none of them can ever be chosen: only the index advances
-                        if (select) candIndex += 56u * (unsigned)nb;
-                    }
-                }
-                if (!poisoned) D4_OR_U32(&st.doneRun, 1u << rn);
-                poisoned = poisoned || outerR;
+        if (item == 0) return !poisoned;
+        // ---- the seed of this runOptimisationsCallbackMulti ------------------------------------------------------------
+        SC wE;
+        if (m == 0) { if (!(seg & SEG_MULTI_H)) return true; wE = wH; }
+        else if (m == 1) { if (!(seg & SEG_MULTI_O)) return true; if (!hasO) return !poisoned; wE = wO; }
+        else if (m == 2) {
+            if (r == 0 && (seg & SEG_FIXED) && blockType != 1) {   // the fixed-code candidate sits between multi(O) and the least seeds
+                long long s2 = 0;
+                const SC F = op_optimise(st, op_to_fixed(st, wH), &s2);
+                cb(st, F);
             }
-            if (!poisoned) D4_OR_U32(&st.doneMulti, 1u << m);
-            poisoned = poisoned || outerM;
+            if (!(seg & SEG_LEAST0)) return !poisoned;
+            wE = op_pass(st, wH, OP_LEAST0);
+        } else { if (!(seg & SEG_LEAST1)) return true; wE = op_pass(st, wH, OP_LEAST1); }
+        if (!wE.ok) { poisoned = true; return false; }
+        // ---- the variant this runOptimisationsCallback works on -------------------------------------------------------
+        SC wX = wE;
+        if (r == 1) wX = op_recode(st, wE);
+        else if (r >= 2) {
+            wX = op_recode_less(st, wE);
+            if (r == 3) {
+                bool full = false;
+                wX = recoded_full(st, wX, &full);
+                if (wX.ok && !full) return !poisoned;
+            }
+        }
+        if (!wX.ok) { poisoned = true; return false; }
+        cb(st, wX);
+        for (int a = 0; a < 3; a++) {
+            SC wY;
+            if (a == 0) {
+                wY = op_hdr(st, wX, HOP_RECODE); cb(st, wY);                                  // post
+                long long sv = 0;
+                const SC o = op_optimise(st, wY, &sv); cb_if_saved(st, o, sv);             // post optimised
+            } else wY = op_pass(st, wX, a == 1 ? OP_LEAST0 : OP_LEAST1);
+            // ---- addOptimisedRecoded(y) ---------------------------------------------------------------------------------
+            // the four bases are only ever read by the trials: their Tab and payload.  Every trial rewrites the header from
+            // the Tab (optimiseBlockDynBlock -> rewriteHeader, DeflateStream.java:184-198), so the header half of
+            // DeflateBlockHuffman.optimise() cannot influence any candidate here and is not run.
+            const int an = (item - 1) * 3 + a;
+            int nb = 0;
+            if (select || !((st.doneAor >> an) & 1)) {   // a base that completed in an earlier sweep asks for nothing
+                const bool outerA = poisoned;
+                poisoned = false;
+                const SC wB0 = op_pass(st, wY, OP_REPLACE);                               // optimiseBlockCopyHelper(toOptimise)
+                const SC wB1 = op_pass(st, op_recode(st, wY), OP_REPLACE);                // optimiseBlockHelper(recodedHuffman(.., false))
+                const SC wPP = op_recode_less(st, wY);                                    // pruned
+                const SC wB2 = op_pass(st, wPP, OP_REPLACE);                              // optimiseBlockCopyHelper(pruned)
+                bool full = false;
+                SC wB3 = recoded_full(st, wPP, &full);                                    // prunedFull
+                if (wB3.ok) {
+                    nb = full ? 4 : 3;
+                    if (full) wB3 = op_pass(st, wB3, OP_REPLACE);
+                    trial_base(st, wB0); trial_base(st, wB1); trial_base(st, wB2);
+                    if (full) trial_base(st, wB3);
+                } else poisoned = true;
+                if (!poisoned) D4_OR_U64(&st.doneAor, 1ull << an);
+                poisoned = poisoned || outerA;
+            }
+            if (a == 0) {
+                const SC t = op_hdr(st, wX, HOP_RECODE_LESS); cb(st, t);                        // pruned header
+                long long sv = 0;
+                const SC o = op_optimise(st, t, &sv); cb_if_saved(st, o, sv);
+                // addOptimisedRecoded(prune) (:431) re-evaluates candidates with exactly the sizes of the sweep on `post`
+                // (both are copies of the same block that differ only in the header, which every base / trial discards),
+                // so under the strict `<` none of them can ever be chosen: only the index advances
+                if (select) candIndex += 56u * (unsigned)nb;
+            }
         }
         return !poisoned;
+    }
+
+    // one item of a discovery sweep (skipped when an earlier sweep of this round completed it) or of the selection sweep
+    D4_HD bool sweep_one(SymState& st, bool sel, unsigned seg, int item) {
+        if (!sel && ((st.doneItem >> item) & 1)) return true;
+        const bool ok = sweep_item(st, sel, seg, item);
+        if (ok && !sel) D4_OR_U32(&st.doneItem, 1u << item);
+        return ok;
+    }
+    // every item in order: one walk over the whole enumeration, whose selection is the reference's
+    D4_HD bool sweep(SymState& st, bool sel, unsigned seg) {
+        bool ok = true;
+        for (int i = 0; i < NITEMS; i++) ok = sweep_one(st, sel, seg, i) && ok;
+        return ok;
+    }
+
+    // ---- items swept apart ------------------------------------------------------------------------------------------------
+    // An item of a selection sweep that runs apart selects inside its own stretch of candidates: indices from 0, best so
+    // far = the value carried into the sweep (begin_item); put_item records the outcome.  join() stitches the records
+    // back in ITEM order, whatever order they were swept in: first strict minimum, indices shifted by the candidates of
+    // the items before.  The result equals the walk over all items in order.
+    D4_HD void begin_item(long long carried) {
+        bestSize = carried; restMin = 0x7fffffffffffffffll; candIndex = 0; bestIndex = 0xffffffffu; bestStored = 0; bestArg = -1;
+    }
+    D4_HD void put_item(ItemRec& e) const {
+        e.bestSize = bestSize; e.restMin = restMin; e.sizeC1 = sizeC1; e.best = best;
+        e.bestIndex = bestIndex; e.candIndex = candIndex; e.bestStored = bestStored; e.bestArg = bestArg;
+    }
+    // returns true when a Huffman candidate of these items became the best
+    D4_HD bool join(const ItemRec* rec) {
+        bool improved = false;
+        unsigned base = candIndex;
+        for (int k = 0; k < NITEMS; k++) {
+            const ItemRec& e = rec[k];
+            if (e.bestIndex != 0xffffffffu && e.bestSize < bestSize) {
+                bestSize = e.bestSize; bestIndex = base + e.bestIndex; bestStored = e.bestStored; bestArg = e.bestArg; best = e.best;
+                improved = !e.bestStored;
+            }
+            if (e.restMin < restMin) restMin = e.restMin;
+            base += e.candIndex;
+        }
+        candIndex = base;
+        sizeC1 = rec[0].sizeC1;   // only the head item sets it
+        return improved;
     }
 };
 

@@ -81,6 +81,7 @@ int host_trial_sizes(const uint8_t* lit, int nlit, const uint8_t* dist, int ndis
 // obvious serial statement of every request kind; the kernels' parallel versions are checked against the oracle on the
 // GPU (tests/test_gpu_parity.py).
 // =====================================================================================================================
+#include <algorithm>
 #include <array>
 #include <cstdio>
 #include <cstdlib>
@@ -321,17 +322,28 @@ struct HostEngine {
         S.trialBits[t] = (unsigned short)best; S.trialArg[t] = (unsigned char)arg; S.trialState[t] = ST_DONE;
         en.trialAll = trialAll.data();
     }
-    // the PENDING entries of the memo tables -> this step's request lists (the kernel does the same with all threads)
+    // the PENDING entries of the memo tables -> this step's request lists (the kernel does the same with all threads).
+    // Passes go in key order: which slot a pass request holds depends on which sweeper claimed it first, and its key does
+    // not, so the ids the executor hands out (and with them the next sweeps) do not depend on the order of the items.
+    std::vector<unsigned long long> reqLog;   // per execute level: a marker, then the sorted keys of its requests
     void collect() {
         S.nqPass = S.nqRec = S.nqHdr = S.nqTrial = 0;
+        std::vector<std::pair<unsigned, int>> pend;
         for (int k = 0; k < PMEMO; k++)
-            if (S.pm[k].key != 0 && S.pm[k].state != ST_DONE && S.nqPass < QPASS) S.qPass[S.nqPass++] = (unsigned short)k;
+            if (S.pm[k].key != 0 && S.pm[k].state != ST_DONE) pend.push_back({S.pm[k].key, k});
+        std::sort(pend.begin(), pend.end());
+        for (const auto& q : pend) if (S.nqPass < QPASS) S.qPass[S.nqPass++] = (unsigned short)q.second;
         for (int k = 0; k < S.nMasks; k++)
             if (S.rc[k].state == ST_PENDING && S.nqRec < QREC) S.qRec[S.nqRec++] = (unsigned short)k;
         for (int k = 0; k < S.nHdrs * 3; k++)
             if (S.hop[k / 3][k % 3] == 0xFFFF && S.nqHdr < QHDR) S.qHdr[S.nqHdr++] = (unsigned short)(((k / 3) << 2) | (k % 3));
         for (int k = 0; k < S.nTabs; k++)
             if (S.trialState[k] == ST_PENDING && S.nqTrial < QTRIAL) S.qTrial[S.nqTrial++] = (unsigned short)k;
+        reqLog.push_back(~0ull);
+        for (const auto& q : pend) reqLog.push_back(q.first);
+        for (int k = 0; k < S.nqRec; k++) reqLog.push_back(1ull << 32 | S.qRec[k]);
+        for (int k = 0; k < S.nqHdr; k++) reqLog.push_back(2ull << 32 | S.qHdr[k]);
+        for (int k = 0; k < S.nqTrial; k++) reqLog.push_back(3ull << 32 | S.qTrial[k]);
     }
     void execute() {
         for (int q = 0; q < S.nqPass; q++) exec_pass(S.qPass[q]);
@@ -352,12 +364,43 @@ struct HostEngine {
         }
     }
     bool segImproved = false, segmentedRound = false;
+    // Order in which the items of a sweep are taken: ORDER_WALK walks them in item order with one enumerator (the
+    // reference's walk; also what a traced selection does); the others sweep every item apart, as the kernel's sweepers
+    // do, and join the selection records in item order.
+    enum { ORDER_WALK = -1, ORDER_FORWARD = 0, ORDER_REVERSE = 1, ORDER_SHUFFLE = 2 };
+    int order = ORDER_FORWARD;
+    unsigned long long shuffleState = 0;
+    std::vector<int> item_order() {
+        std::vector<int> o(NITEMS);
+        for (int i = 0; i < NITEMS; i++) o[i] = order == ORDER_REVERSE ? NITEMS - 1 - i : i;
+        if (order == ORDER_SHUFFLE)
+            for (int i = NITEMS - 1; i > 0; i--) {   // Fisher-Yates over a 64-bit LCG: a new permutation every sweep
+                shuffleState = shuffleState * 6364136223846793005ull + 1442695040888963407ull;
+                std::swap(o[i], o[(int)((shuffleState >> 33) % (unsigned long long)(i + 1))]);
+            }
+        return o;
+    }
+    bool sweep_apart(bool sel, unsigned seg) {
+        bool ok = true;
+        ItemRec rec[NITEMS];
+        const long long carried = en.bestSize;
+        for (int item : item_order()) {
+            Enumer w = en;
+            w.trace = nullptr;
+            if (sel) w.begin_item(carried);
+            ok = w.sweep_one(S, sel, seg, item) && ok;
+            if (w.internalError) en.internalError = w.internalError;
+            if (sel) w.put_item(rec[item]);
+        }
+        if (sel) segImproved = en.join(rec);
+        return ok;
+    }
     bool run_segment(unsigned seg) {
-        S.doneMulti = 0; S.doneRun = 0; S.doneAor = 0;
+        S.doneItem = 0; S.doneAor = 0;
+        const bool walk = order == ORDER_WALK;
         for (int it = 0;; it++) {
             nSweeps++;
-            bool done = true;
-            for (int m = 0; m < 4; m++) done = en.sweep(S, false, seg, m, m + 1) && done;   // one seed per sweeping thread
+            const bool done = walk ? en.sweep(S, false, seg) : sweep_apart(false, seg);
             if (S.overflow) return false;
             collect();
             const bool nothing = S.nqPass + S.nqRec + S.nqHdr + S.nqTrial == 0;
@@ -366,10 +409,12 @@ struct HostEngine {
             execute();
             if (S.overflow) return false;
         }
-        const unsigned before = en.bestIndex;
-        en.sweep(S, true, seg);
-        segImproved = en.bestIndex != before && !en.bestStored;
-        if (en.internalError || en.poisoned) err = 16;
+        if (walk || en.trace) {
+            const unsigned before = en.bestIndex;
+            if (!en.sweep(S, true, seg)) err = 16;
+            segImproved = en.bestIndex != before && !en.bestStored;
+        } else if (!sweep_apart(true, seg)) err = 16;
+        if (en.internalError) err = 16;
         return true;
     }
     void optimise_block(long long storedSize, bool forceSegmented) {
@@ -460,6 +505,24 @@ int host_engine_round(void* p, long long storedSize, int forceSegmented, long lo
     if (getenv("D4_HOST_DCSTATS")) fprintf(stderr, "dcstats builds %lld avg_changed_bytes %.2f touched_frac %.3f flips %lld byte_updates_per_build %.0f matches %lld\n", e->statBuilds, e->statBuilds ? (double)e->statChanged / e->statBuilds : 0.0, e->statMatches ? (double)e->statTouched / e->statMatches : 0.0, e->statFlip, e->statBuilds ? (double)e->statBytesTouched / e->statBuilds : 0.0, e->statBuilds ? e->statMatches / e->statBuilds : 0);
     if (traceN) *traceN = e->traceN;
     return e->err;
+}
+// order of the items of every following sweep (HostEngine::ORDER_*); seed: the shuffle's
+void host_engine_order(void* p, int order, unsigned long long seed) {
+    HostEngine* e = (HostEngine*)p;
+    e->order = order; e->shuffleState = seed;
+}
+// selection state after the last round: {bestSize, bestIndex, bestStored, bestArg, restMin, sizeC1, candIndex}
+void host_engine_selection(void* p, long long* out) {
+    const Enumer& en = ((HostEngine*)p)->en;
+    out[0] = en.bestSize; out[1] = en.bestIndex; out[2] = en.bestStored; out[3] = en.bestArg; out[4] = en.restMin;
+    out[5] = en.sizeC1; out[6] = en.candIndex;
+}
+// the request log since the block was loaded: per execute level ~0, then its requests (pass keys; 1 << 32 | mask id of a
+// recode; 2 << 32 | hid << 2 | op of a header op; 3 << 32 | table id of a trial).  Returns its length.
+size_t host_engine_reqlog(void* p, unsigned long long* buf, size_t cap) {
+    const auto& l = ((HostEngine*)p)->reqLog;
+    for (size_t k = 0; k < l.size() && k < cap; k++) buf[k] = l[k];
+    return l.size();
 }
 // the winner becomes the block (the next optimiseBlock call of DeflateStream.optimise's loop)
 void host_engine_advance(void* p, int keepPools) { ((HostEngine*)p)->advance_to_best(keepPools != 0); }
